@@ -3,7 +3,7 @@
 (SURVEY §8d) on synthetic graphs of the shapes BASELINE.json names, through the reference's own
 layer API (layer_dict[name](dim_in, dim_out, bias) + forward(batch) + backward).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.
   value     device-resident: inputs and the graph layout already in HBM, K timed steps (CUDA events)
@@ -291,6 +291,27 @@ def _timed_steps(fn, steps, warmup, sync_all, max_over_ranks):
     return max_over_ranks(s.elapsed_time(e)) / steps
 
 
+DUMP_BYTES = 60_000_000   # --dump-outputs writes at most this much (array data; each .npy header adds 128 bytes)
+
+
+def dump_outputs(path, rows=None, whole=None):
+    """--dump-outputs: write every array as path/<name>.npy in float32 (float64 stays float64).  ``whole`` arrays are
+    written whole; the per-node arrays in ``rows`` keep one seeded sample of their rows, as many as fit DUMP_BYTES, so that
+    two builds run with the same arguments write files that compare element for element."""
+    rows, whole = rows or {}, whole or {}
+    host = lambda t: t.detach().cpu().numpy() if t.dtype == torch.float64 else t.detach().float().cpu().numpy()
+    out = {name: host(t) for name, t in whole.items()}
+    if rows:
+        n = next(iter(rows.values())).size(0)
+        row_bytes = sum(t[0].numel() * (8 if t.dtype == torch.float64 else 4) for t in rows.values())
+        keep = min(n, (DUMP_BYTES - sum(a.nbytes for a in out.values())) // row_bytes)
+        pick = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out.update({name: host(t[pick.to(t.device)]) for name, t in rows.items()})
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
 def cpu_cycles_baseline(seconds):
     """The reference algorithm itself (identity.py:25-35: dense A_hat, k-1 dense matmuls) on BA graphs of growing size; at
     1M nodes it is infeasible (n^2 floats = 4 TB)."""
@@ -414,6 +435,8 @@ def run_aux(args, spec, dev, rank=0, world=1):
         launches0 = ops.launch_count()
         with clocks:
             ms = _timed_steps(one_block, args.steps, args.warmup, sync_all, max_over_ranks)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, whole={'diag': out})   # the last timed block's diag(A_hat^1..k)
         launches = int(sum_over_ranks((ops.launch_count() - launches0) * args.steps // (args.steps + args.warmup)))
         hops = (k + 1) // 2
         slots = csr.num_slots
@@ -473,6 +496,7 @@ def run_aux(args, spec, dev, rank=0, world=1):
             stages = [layer_dict['ginidconv'](dims[i], dims[i + 1], bias=True).to(dev) for i in range(nl)]
             x = gen_features(n_out, dims[0], dev, seed=rank)
         gy = gen_features(n_out, dims[-1], dev, seed=7 + rank)
+        keep = {} if args.dump_outputs else None   # the latest step's results, held only to be dumped
 
         def step():
             for l in stages:
@@ -487,8 +511,14 @@ def run_aux(args, spec, dev, rank=0, world=1):
             if world > 1:
                 for l in stages:
                     parallel.allreduce_grads(l)
+            if keep is not None:
+                keep.update(rows={'out': b.node_feature.detach(), 'grad_x': h.grad},
+                            whole={f'grad_{i}.{k}': p.grad for i, l in enumerate(stages)
+                                   for k, p in l.named_parameters() if p.grad is not None})
         launches0 = ops.launch_count()
         ms = _timed_steps(step, args.steps, args.warmup, sync_all, max_over_ranks)
+    if keep is not None:
+        dump_outputs(args.dump_outputs, **keep)
     launches = int(sum_over_ranks((ops.launch_count() - launches0) * args.steps // (args.steps + args.warmup)))
     slots_per_layer = e_out + (n_out if cfg_a else 0)      # gcnidconv adds the remaining self loops
     ef_rank = sum(slots_per_layer * (dims[i + 1] if cfg_a else dims[i]) * 2 for i in range(nl))
@@ -664,6 +694,8 @@ def run_ours(args, spec, rank, world, dev):
                 return prm.grad
         return next(layer.parameters()).grad
 
+    keep = {} if args.dump_outputs else None   # the latest step's results, held only until the timed steps are dumped
+
     def step(x_dev, ei_dev, playout=None):
         layer.zero_grad(set_to_none=True)
         # the layer input needs its gradient: message-passing layers sit behind pre_mp / earlier layers
@@ -675,7 +707,11 @@ def run_ours(args, spec, rank, world, dev):
             parallel.allreduce_grads(layer)
         else:
             b = layer(Batch(x_dev, ei_dev, ids))
-            b.node_feature.backward(gy_loc)
+            y = b.node_feature
+            y.backward(gy_loc)
+        if keep is not None:
+            keep.update(rows={'out': y.detach(), 'grad_x': x_dev.grad},
+                        whole={'grad_' + k: p.grad for k, p in layer.named_parameters() if p.grad is not None})
         return bias_grad()
 
     t0 = time.time()
@@ -741,6 +777,9 @@ def run_ours(args, spec, rank, world, dev):
     launches = int(sum_over_ranks(ops.launch_count() - launches0))
     ms = max_over_ranks(start.elapsed_time(end)) / args.steps
     clocks.__exit__(None, None, None)
+    if keep is not None:
+        dump_outputs(args.dump_outputs, **keep)
+        keep = None
     ef, f_agg = edge_feat_per_step(name, n, slots, fin, fout)
     value = ef / (ms * 1e-3) / 1e9
 
@@ -1096,10 +1135,18 @@ def main():
     ap.add_argument('--gather-dtype', default='f32', choices=['f32', 'bf16'],
                     help="storage of the aggregation's gathered operand: f32 (reference arithmetic, the default and "
                          "the headline) or bf16 (the north star's 1e-2 mode; single GPU)")
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (layer output, input gradient, '
+                         'parameter gradients; a seeded sample of the rows of per-node arrays, %d bytes at most) as '
+                         'DIR/<name>.npy, to compare two builds output for output (single GPU)' % DUMP_BYTES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     spec = WORKLOADS[args.workload]
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
+    if args.dump_outputs and (world > 1 or args.impl == 'reference'):
+        ap.error('--dump-outputs dumps the single-GPU timed path (--impl ours, one process)')
     if args.impl == 'reference':
         if spec.get('aux'):
             raise SystemExit('--impl reference covers the layer workloads')

@@ -138,6 +138,32 @@ def test_bench_generators_are_seeded_and_well_formed():
     assert bench.spmm_bytes(10, 100, 8, False, gather_bytes=2) == 100 * 8 * 2 + 10 * 8 * 4 + 100 * 4 + 11 * 4
 
 
+def test_bench_dump_outputs_keeps_one_seeded_row_sample_within_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every per-node array keeps the same rows, the same ones on every call; whole arrays are
+    written whole; float32 on disk unless float64; the array data fits DUMP_BYTES."""
+    import numpy as np
+
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 40_000)
+    g = torch.Generator().manual_seed(0)
+    out = torch.randn(1000, 8, generator=g)
+    rows = {'out': out, 'grad_x': out[:, :4].double() * 2}      # 64 bytes a row: (40000 - 128) // 64 = 623 rows
+    whole = {'grad_w': torch.randn(4, 8, generator=g)}
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), rows=rows, whole=whole)
+    a = {f[:-4]: np.load(tmp_path / 'a' / f) for f in os.listdir(tmp_path / 'a')}
+    b = {f[:-4]: np.load(tmp_path / 'b' / f) for f in os.listdir(tmp_path / 'b')}
+    assert sorted(a) == ['grad_w', 'grad_x', 'out'] and all(np.array_equal(a[k], b[k]) for k in a)
+    assert a['out'].shape == (623, 8) and a['out'].dtype == np.float32 and a['grad_x'].dtype == np.float64
+    assert np.array_equal(a['grad_x'], a['out'][:, :4].astype(np.float64) * 2)        # the same rows in every array
+    assert np.array_equal(a['grad_w'], whole['grad_w'].numpy())
+    assert sum(v.nbytes for v in a.values()) <= 40_000
+    picked = {tuple(r) for r in a['out'].tolist()}
+    assert len(picked) == 623 and picked <= {tuple(r) for r in out.tolist()}
+    bench.dump_outputs(str(tmp_path / 'c'), rows={'out': out[:10]})                  # small arrays are written whole
+    assert np.array_equal(np.load(tmp_path / 'c' / 'out.npy'), out[:10].numpy())
+
+
 def test_every_environment_switch_is_documented():
     """INTEGRATION.md §7 lists every GG_* variable the package, the C-ABI library sources and bench.py read."""
     import os
