@@ -7,7 +7,8 @@ products-shaped graph.  SURVEY §8(d) prescribes edge chunking for that size.  T
 slices of the edge list and spell the backward out by hand — exactly the ops autograd would run (index_add_'s backward is
 an index_select of the gradient, the scale's backward is the same scale, index_select's backward is an index_add_) — so
 that no per-edge tensor outlives its chunk.  ``tests/test_oracle_golden.py`` pins them against ``oracle/layers.py`` +
-autograd on small inputs.  They are the CPU arm of ``bench.py`` at full size (kind "port").
+autograd on small inputs.  They are the CPU arm of ``bench.py`` at full size (kind "port"), and they run wherever their
+inputs live: in float64 on the GPU they are the reference of ``tests/test_fullsize_step_parity_gpu.py``.
 """
 import torch
 import torch.nn.functional as F
@@ -47,7 +48,8 @@ def sageconv_step(x, edge_index, w_l, b_l, w_r, gy, chunk=1 << 22):
     """-> (out, dx, dw_l, db_l, dw_r) of oracle.layers.sageconv (weights are nn.Linear [out, in])."""
     n = x.size(0)
     src, tgt = edge_index
-    cnt = torch.zeros(n, dtype=x.dtype).index_add_(0, tgt, torch.ones(tgt.numel(), dtype=x.dtype)).clamp(min=1)
+    cnt = torch.zeros(n, dtype=x.dtype, device=x.device).index_add_(0, tgt, torch.ones(tgt.numel(), dtype=x.dtype,
+                                                                             device=x.device)).clamp(min=1)
     mean = _scatter_messages(torch.zeros_like(x), x, src, tgt, None, chunk) / cnt.view(-1, 1)
     out = F.linear(mean, w_l, b_l) + F.linear(x, w_r)
     gmean = (gy @ w_l) / cnt.view(-1, 1)
@@ -55,9 +57,10 @@ def sageconv_step(x, edge_index, w_l, b_l, w_r, gy, chunk=1 << 22):
     return out, dx, gy.t() @ mean, (gy.sum(0) if b_l is not None else None), gy.t() @ x
 
 
-def gatconv_step(x, edge_index, weight, att, bias, gy, negative_slope=0.2, chunk=1 << 22):
-    """-> (out, dx, dweight, datt, dbias) of oracle.layers.gatconv with heads = 1.  Per-edge SCALARS (logits, alpha) are
-    kept whole ([E] floats); every [E, C] tensor is chunked.  The reference additionally materialises cat([x_i, x_j])
+def gatconv_step(x, edge_index, weight, att, bias, gy, negative_slope=0.2, chunk=1 << 22, return_alpha=False):
+    """-> (out, dx, dweight, datt, dbias) of oracle.layers.gatconv with heads = 1; with ``return_alpha`` also alpha [E']
+    over the edge list the layer aggregates (self loops removed, then one per node appended).  Per-edge SCALARS (logits,
+    alpha) are kept whole ([E] floats); every [E, C] tensor is chunked.  The reference additionally materialises cat([x_i, x_j])
     [E, 2C] (idconv.py:323-326): this port is cheaper than the reference's own op sequence."""
     n, c = x.size(0), weight.size(1)
     ei, _ = U.remove_self_loops(edge_index)
@@ -76,12 +79,13 @@ def gatconv_step(x, edge_index, weight, att, bias, gy, negative_slope=0.2, chunk
     dalpha = torch.empty_like(alpha)
     for a, b in _chunks(src.numel(), chunk):
         dalpha[a:b] = (gy.index_select(0, tgt[a:b]) * h.index_select(0, src[a:b])).sum(1)
-    dot = torch.zeros(n, dtype=x.dtype).index_add_(0, tgt, alpha * dalpha)
+    dot = torch.zeros(n, dtype=x.dtype, device=x.device).index_add_(0, tgt, alpha * dalpha)
     dlz = alpha * (dalpha - dot[tgt])
     dz = dlz * torch.where(z > 0, torch.ones_like(z), torch.full_like(z, negative_slope))
-    ds_t = torch.zeros(n, dtype=x.dtype).index_add_(0, tgt, dz)
-    ds_s = torch.zeros(n, dtype=x.dtype).index_add_(0, src, dz)
+    ds_t = torch.zeros(n, dtype=x.dtype, device=x.device).index_add_(0, tgt, dz)
+    ds_s = torch.zeros(n, dtype=x.dtype, device=x.device).index_add_(0, src, dz)
     dh = _scatter_messages(torch.zeros_like(h), gy, tgt, src, alpha, chunk)
     dh += ds_t.view(-1, 1) * a_t + ds_s.view(-1, 1) * a_s
     datt = torch.cat([h.t() @ ds_t, h.t() @ ds_s]).view_as(att)
-    return out, dh @ weight.t(), x.t() @ dh, datt, (gy.sum(0) if bias is not None else None)
+    res = (out, dh @ weight.t(), x.t() @ dh, datt, (gy.sum(0) if bias is not None else None))
+    return res + (alpha,) if return_alpha else res

@@ -4,6 +4,8 @@
 (``norm`` at :7-22, remaining self loops, degree over edge_index[0]), densified, and
 diag(A_hat^p) for p = 1..k by repeated dense matmul.  ``closed_walks`` is the integer variant the
 north star names (diag(A^p), exact int64) — the reference itself never computes it (SURVEY D2).
+``diag_powers_sparse`` is the same A_hat's diagonal powers for chosen source nodes without densifying, for graphs far
+past the dense form's reach (on the device of the edge list).
 """
 import numpy as np
 import torch
@@ -21,6 +23,27 @@ def compute_identity(edge_index, n, k, dtype=torch.float32):
         power = power @ adj
         diag_all.append(torch.diag(power))
     return torch.stack(diag_all, dim=1)
+
+
+def diag_powers_sparse(edge_index, n, k, sources, chunk=1 << 21):
+    """[len(sources), k] float64: diag(A_hat^p)[sources] for p = 1..k with the A_hat of ``compute_identity``, by k hops
+    V <- A_hat V from the sources' unit columns (gather / scale / index_add_ over edge chunks)."""
+    ei, value = gcn_norm_src(edge_index, n, torch.float64)
+    row, col = ei
+    dev = edge_index.device
+    s = torch.as_tensor(sources, device=dev).long()
+    cols = torch.arange(s.numel(), device=dev)
+    v = torch.zeros((n, s.numel()), dtype=torch.float64, device=dev)
+    v[s, cols] = 1.0
+    out = torch.empty((s.numel(), k), dtype=torch.float64, device=dev)
+    for p in range(k):
+        nxt = torch.zeros_like(v)
+        for a in range(0, row.numel(), chunk):
+            b = min(row.numel(), a + chunk)
+            nxt.index_add_(0, row[a:b], v.index_select(0, col[a:b]) * value[a:b].view(-1, 1))
+        v = nxt
+        out[:, p] = v[s, cols]
+    return out
 
 
 def closed_walks(edge_index, n, k):

@@ -21,7 +21,7 @@ def id_transform(x, ids, weight, weight_id):
 
 def gcn_norm_src(edge_index, num_nodes, dtype, improved=False):
     """ref: idconv.py:132-148 / identity.py:7-22 — remaining self loops, degree over edge_index[0]."""
-    w = torch.ones(edge_index.size(1), dtype=dtype)
+    w = torch.ones(edge_index.size(1), dtype=dtype, device=edge_index.device)
     edge_index, w = U.add_remaining_self_loops(edge_index, w, 2 if improved else 1, num_nodes)
     row, col = edge_index
     deg = U.scatter_add(w, row, 0, num_nodes)
@@ -32,7 +32,7 @@ def gcn_norm_src(edge_index, num_nodes, dtype, improved=False):
 
 def gcn_norm_tgt(edge_index, num_nodes, dtype):
     """PyG >= 1.6 ``gcn_norm`` (used by pyg.nn.GCNConv, ref: layer.py:138): degree over edge_index[1]."""
-    w = torch.ones(edge_index.size(1), dtype=dtype)
+    w = torch.ones(edge_index.size(1), dtype=dtype, device=edge_index.device)
     edge_index, w = U.add_remaining_self_loops(edge_index, w, 1, num_nodes)
     row, col = edge_index
     deg = U.scatter_add(w, col, 0, num_nodes)

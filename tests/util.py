@@ -36,7 +36,9 @@ def powerlaw_graph(seed, n, avg_deg, max_deg=None, exponent=2.1):
 
 
 def rel_err(a, b):
-    """max |a-b| / max(|b|, tiny): the norm-wise relative error used for every fp parity check."""
+    """max |a-b| / max(|b|, tiny): the norm-wise relative error used for every fp parity check.  Not enough alone where the
+    rows or columns differ in scale (hub rows of a sum aggregation, high powers of compute_identity): the largest one sets
+    the denominator and hides errors in the small ones; bound each element by its own scale there as well."""
     a = torch.as_tensor(a, dtype=torch.float64).cpu()
     b = torch.as_tensor(b, dtype=torch.float64).cpu()
     assert a.shape == b.shape, (a.shape, b.shape)
