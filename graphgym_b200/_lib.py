@@ -71,6 +71,17 @@ SIGNATURES = {
     "gg_spmm_sell_f32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64, c_ptr,
                                  c_i64, c_ptr, c_int, c_i64, c_i64, c_i64, c_int, c_ptr, c_i64, c_f32, c_ptr, c_ptr, c_ptr,
                                  c_ptr, c_ptr, c_ptr, c_size, c_int, c_ptr]),
+    "gg_spmm_sell_max_workspace_bytes": (c_size, [c_i64, c_i64]),
+    "gg_spmm_sell_max_f32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64,
+                                     c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_ptr, c_i64, c_f32, c_ptr, c_ptr, c_size,
+                                     c_int, c_ptr]),
+    "gg_spmm_sell_max_bwd_f32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr,
+                                         c_i64, c_ptr, c_i64, c_i64, c_i64, c_f32, c_ptr, c_i64, c_ptr, c_size, c_int,
+                                         c_ptr]),
+    "gg_spmm_row_max_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_ptr,
+                                    c_i64, c_f32, c_ptr, c_ptr]),
+    "gg_spmm_row_max_bwd_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_f32,
+                                        c_ptr, c_i64, c_ptr]),
     "gg_cast_f32_bf16": (c_int, [c_ptr, c_i64, c_i64, c_i64, c_ptr, c_i64, c_ptr]),
     "gg_spmm_mp_bf16": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64,
                                 c_int, c_ptr, c_i64, c_f32, c_ptr, c_ptr, c_size, c_int, c_ptr]),

@@ -3,7 +3,8 @@ primitives (SURVEY §8f item 4).
 
 GeneralConvLayer (ref: graphgym/contrib/layer/generalconv.py:12-113): h = x W; optional GCN normalisation
 (``cfg.gnn.normalize_adj``: remaining self loops, degree over edge_index[0]); aggregate with ``cfg.gnn.agg``; then the self
-message ``cfg.gnn.self_msg``: 'none' | 'add' (+ h) | 'concat' (+ x W_self); + bias.
+message ``cfg.gnn.self_msg``: 'none' | 'add' (+ h) | 'concat' (+ x W_self); + bias.  ``agg = 'max'``: torch_scatter's
+scatter_max (empty rows 0), the gradient to the first in-edge that reaches each column's maximum.
 SAGEConvLayer (ref: graphgym/contrib/layer/sageinitconv.py:12-102, used with concat=True by ``sageinitconv``):
 [x || mean_j x_j] W + bias, no self loops.
 """
@@ -22,8 +23,9 @@ from graphgym_b200.register import register_layer
 class GeneralConvLayer(nn.Module):
     def __init__(self, in_channels, out_channels, improved=False, cached=False, bias=True, **kwargs):
         super().__init__()
-        if cfg.gnn.agg not in ('add', 'mean'):
-            raise NotImplementedError("cfg.gnn.agg = {!r}: 'add' and 'mean' are on the accelerated path".format(cfg.gnn.agg))
+        if cfg.gnn.agg not in ('add', 'mean', 'max'):
+            raise NotImplementedError("cfg.gnn.agg = {!r}: 'add', 'mean' and 'max' are on the accelerated path".format(
+                cfg.gnn.agg))
         if improved:
             raise NotImplementedError('improved=True is never set by the GraphGym wrappers (ref: layer.py:189-191)')
         self.in_channels, self.out_channels = in_channels, out_channels
@@ -53,9 +55,9 @@ class GeneralConvLayer(nn.Module):
         h = F_.seg_linear([x], [self.weight], [(0, 0, False)])
         if self.normalize:
             layout = get_layout(edge_index, n, ops.LOOPS_ADD_REMAINING)
-            kind = 'gcn_src_mean' if self.aggr == 'mean' else 'gcn_src'
+            kind = {'add': 'gcn_src', 'mean': 'gcn_src_mean', 'max': 'gcn_src_max'}[self.aggr]
         else:
-            layout, kind = get_layout(edge_index, n, ops.LOOPS_KEEP), ('mean' if self.aggr == 'mean' else 'sum')
+            layout, kind = get_layout(edge_index, n, ops.LOOPS_KEEP), {'add': 'sum', 'mean': 'mean', 'max': 'max'}[self.aggr]
         if self.self_msg == 'none':
             return F_.aggregate(h, layout, kind, 0.0, self.bias)
         if self.self_msg == 'add':       # x_msg (+ bias, added in update) + x, x = the transformed features

@@ -1,7 +1,7 @@
 """Differentiable building blocks of the layers: each one is a ``torch.autograd.Function`` whose
 forward AND backward are ``gg_*`` kernels (no torch math on the path).
 
-  aggregate    CSR SpMM forward, CSC SpMM backward            (SURVEY §8a row 4)
+  aggregate    CSR SpMM forward, CSC SpMM backward            (SURVEY §8a row 4); max: arg-max forward, masked CSC sum
   seg_linear   multi-segment dense transform with ID weights  (SURVEY §8a row 9)
   gather_rows / scatter_add_rows   the M-row ID branch of GIN-ID (ref: idconv.py:372-375)
 """
@@ -42,10 +42,47 @@ class _Aggregate(torch.autograd.Function):
         return gx, None, None, None, gb, None, (g if ctx.has_residual else None)
 
 
+class _AggregateMax(torch.autograd.Function):
+    """out[i] = max_{j->i} w_ji x[j] (0 without in-edges) + self_scale * x[i] + residual[i] + bias; the gradient of the
+    max goes to the first in-edge (in edge order) that reaches it, per column."""
+
+    @staticmethod
+    def forward(ctx, x, layout, kind, self_scale, bias, residual=None):
+        w_fwd, _ = layout.weights(kind)
+        x = x.contiguous()
+        if residual is not None:
+            if self_scale != 0.0:
+                raise ValueError("aggregate: residual excludes self_scale")
+            out, arg = ops.spmm_max(layout.csr, x, w_fwd, residual.contiguous(), 1.0, bias)
+        else:
+            out, arg = ops.spmm_max(layout.csr, x, w_fwd, x if self_scale != 0.0 else None, self_scale, bias)
+        ctx.layout, ctx.kind, ctx.self_scale = layout, kind, self_scale
+        ctx.has_bias, ctx.has_residual = bias is not None, residual is not None
+        ctx.save_for_backward(arg)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        g = g.contiguous()
+        gx = gb = None
+        if ctx.needs_input_grad[0]:
+            (arg,) = ctx.saved_tensors
+            _, w_bwd = ctx.layout.weights(ctx.kind)
+            gx = ops.spmm_max_bwd(ctx.layout.csc, ctx.layout.csc2csr, g, arg, w_bwd, ctx.self_scale)
+        if ctx.has_bias and ctx.needs_input_grad[4]:
+            gb = ops.colsum(g)
+        return gx, None, None, None, gb, (g if ctx.has_residual else None)
+
+
 def aggregate(x, layout, kind="sum", self_scale=0.0, bias=None, residual=None):
     """out[i] = reduce_{j->i} w_ji x[j] + self_scale * x[i] + residual[i] + bias.  ``cfg.b200.gather_dtype = 'bf16'``
-    stores the gathered operand in bf16 (forward and backward) when the width allows it (f % 8 == 0, f <= 256)."""
+    stores the gathered operand in bf16 (forward and backward) when the width allows it (f % 8 == 0, f <= 256).
+    Kinds ending in 'max' reduce with a max (fp32 only)."""
     from .config import cfg
+    if kind.endswith("max"):
+        if cfg.b200.gather_dtype == "bf16":
+            raise NotImplementedError("cfg.b200.gather_dtype = 'bf16' has no max aggregation (kind {!r})".format(kind))
+        return _AggregateMax.apply(x, layout, kind, float(self_scale), bias, residual)
     half = cfg.b200.gather_dtype == "bf16" and ops.bf16_gather_ok(x.size(1))
     return _Aggregate.apply(x, layout, kind, float(self_scale), bias, half, residual)
 

@@ -65,9 +65,11 @@ class GraphLayout:
         'gcn_src'  D^-1/2 A D^-1/2 with the degree summed over edge_index[0] (ref: idconv.py:143-148)
         'gcn_tgt'  same with the degree summed over edge_index[1] (PyG >= 1.6 GCNConv, layer.py:138)
         'gcn_src_mean'  'gcn_src' weights reduced with a mean over the target's in-edges
+        'max'      no weights, max over the in-edges (functional._AggregateMax)
+        'gcn_src_max'   'gcn_src' weights, max over the target's normalised messages
         """
         if kind not in self._weights:
-            if kind == "sum":
+            if kind in ("sum", "max"):
                 w = (None, None)
             elif kind == "mean":
                 indeg = ops.segment_degree(self.csr)
@@ -81,6 +83,9 @@ class GraphLayout:
                 # One elementwise product per layout (layout-build level, cached).
                 w_csr, w_csc = self.weights("gcn_src")
                 w = (w_csr, w_csc * ops.mean_weights(self.csc, ops.segment_degree(self.csr)))
+            elif kind == "gcn_src_max":
+                # MessagePassing(aggr='max') over the normalised messages: the backward scales by the same w_e
+                w = self.weights("gcn_src")
             else:
                 raise KeyError(kind)
             self._weights[kind] = w

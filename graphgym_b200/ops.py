@@ -311,6 +311,16 @@ def sell_layout(csr):
     return csr._sell
 
 
+def _sell_hub_idx(sl, n_src, f, flags):
+    """(idx, flags) of a sliced-ELL aggregation call gathering ``n_src`` rows of width ``f``."""
+    # hub hint: only when the gathered matrix is (much) larger than what the hint keeps resident
+    if SELL_HUB_BYTES and f >= SELL_HUB_MIN_F and n_src * f * 4 > 2 * SELL_HUB_BYTES and (flags & 4):
+        # hub count in powers of two: the hint array is rebuilt only when the width class changes
+        hubs = 1 << max(10, (SELL_HUB_BYTES // (4 * f)).bit_length() - 1)
+        return sl.idx_hint(hubs), flags | 8
+    return sl.idx, flags
+
+
 def _spmm_sell(csr, x, ldx, x_ptr, w_slot, reduce, x_self, ld_self, self_scale, bias, r1, out, ldo, out_peers):
     sl = sell_layout(csr)
     L = lib()
@@ -318,17 +328,96 @@ def _spmm_sell(csr, x, ldx, x_ptr, w_slot, reduce, x_self, ld_self, self_scale, 
     ws_bytes = int(L.gg_spmm_sell_workspace_bytes(sl.partial_rows, f))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
     peers = (out_peers._arr, len(out_peers.ptrs), out_peers.rows_per_rank) if out_peers is not None else (None, 1, max(csr.num_nodes, 1))
-    idx, flags = sl.idx, _spmm_flags()
-    # hub hint: only when the gathered matrix is (much) larger than what the hint keeps resident
-    if SELL_HUB_BYTES and f >= SELL_HUB_MIN_F and x.size(0) * f * 4 > 2 * SELL_HUB_BYTES and (flags & 4):
-        # hub count in powers of two: the hint array is rebuilt only when the width class changes
-        hubs = 1 << max(10, (SELL_HUB_BYTES // (4 * f)).bit_length() - 1)
-        idx, flags = sl.idx_hint(hubs), flags | 8
+    idx, flags = _sell_hub_idx(sl, x.size(0), f, _spmm_flags())
     check(L.gg_spmm_sell_f32(_ptr(sl.chunk_ptr), sl.chunks, _ptr(idx), _ptr(sl.weights(w_slot)), _ptr(sl.vdst),
                              _ptr(csr.rowptr), _ptr(sl.hub_rows), _ptr(sl.hub_pptr), sl.hubs, sl.partial_rows, x_ptr, ldx,
                              _ptr(out), ldo, peers[0], peers[1], peers[2], csr.num_nodes, f, reduce, _ptr(x_self), ld_self,
                              float(self_scale), _ptr(bias), _ptr(r1[0]), _ptr(r1[1]), _ptr(r1[2]), _ptr(r1[3]), _ptr(ws),
                              ws_bytes, flags, _stream()), "gg_spmm_sell_f32")
+
+
+def _al16(t):
+    return t is None or t.data_ptr() % 16 == 0
+
+
+def spmm_max(csr, x, w_slot=None, x_self=None, self_scale=0.0, bias=None, algo=None):
+    """Max aggregation -> (out [n, f], arg int32 [n, f]):
+    out[i,:] = max_{s in segment i} w[s]*x[nbr[s],:] (0 for an empty segment) + self_scale*x_self[i,:] + bias;
+    arg[i,c] = the first slot (in slot order) reaching the maximum, -1 for an empty segment (csrc/spmm_max.cu).
+    The sliced-ELL kernel runs where ``spmm`` would run its sliced-ELL path (f % 4 == 0, 16-byte rows, n + slots >=
+    2**14; wider rows as column tiles of 128), the warp-per-row kernel otherwise.  ``algo`` ('sell' | 'row') overrides the
+    choice for this call."""
+    _need_cuda(x, w_slot, x_self, bias, csr.rowptr)
+    x, ldx = _rows(x, "x")
+    n, f = csr.num_nodes, x.size(1)
+    dev = x.device
+    out = torch.empty((n, f), dtype=torch.float32, device=dev)
+    arg = torch.empty((n, f), dtype=torch.int32, device=dev)
+    if n == 0 or f == 0:
+        return out, arg
+    ld_self = 0
+    if x_self is not None:
+        x_self, ld_self = _rows(x_self, "x_self")
+    if bias is not None:
+        bias = bias.contiguous()
+    L = lib()
+    aligned = f % 4 == 0 and ldx % 4 == 0 and _al16(x) and _al16(bias) and (x_self is None or (ld_self % 4 == 0 and _al16(x_self)))
+    if algo is None:
+        algo = "sell" if aligned and n + csr.num_slots >= 1 << 14 else "row"
+    if algo == "sell":
+        if not aligned:
+            raise ValueError("spmm_max: the sliced-ELL kernel needs f % 4 == 0 and 16-byte aligned rows")
+        sl = sell_layout(csr)
+        ws_bytes = int(L.gg_spmm_sell_max_workspace_bytes(sl.partial_rows, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        idx, flags = _sell_hub_idx(sl, x.size(0), min(f, 128), _spmm_flags())
+        check(L.gg_spmm_sell_max_f32(_ptr(sl.chunk_ptr), sl.chunks, _ptr(idx), _ptr(sl.slot_of), _ptr(sl.weights(w_slot)),
+                                     _ptr(sl.vdst), _ptr(sl.hub_rows), _ptr(sl.hub_pptr), sl.hubs, sl.partial_rows, _ptr(x),
+                                     ldx, _ptr(out), f, _ptr(arg), f, n, f, _ptr(x_self), ld_self, float(self_scale),
+                                     _ptr(bias), _ptr(ws), ws_bytes, flags, _stream()), "gg_spmm_sell_max_f32")
+    elif algo == "row":
+        check(L.gg_spmm_row_max_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(w_slot), _ptr(x), ldx, _ptr(out), f, _ptr(arg), f,
+                                    n, f, _ptr(x_self), ld_self, float(self_scale), _ptr(bias), _stream()),
+              "gg_spmm_row_max_f32")
+    else:
+        raise ValueError(f"spmm_max: algo={algo!r}")
+    return out, arg
+
+
+def spmm_max_bwd(csc, csc2csr, g, arg, w_slot_csc=None, self_scale=0.0, algo=None):
+    """Backward of ``spmm_max`` wrt x: dx[j,:] = sum over the CSC slots t of row j whose edge won its column
+    (arg[target, c] == CSR slot of the edge) of w_csc[t] * g[target, :], + self_scale * g[j, :].  Path choice as in
+    ``spmm_max``."""
+    _need_cuda(g, arg, w_slot_csc, csc.rowptr)
+    g, ldg = _rows(g, "g")
+    arg = arg.contiguous()
+    n, f = csc.num_nodes, g.size(1)
+    dev = g.device
+    dx = torch.empty((n, f), dtype=torch.float32, device=dev)
+    if n == 0 or f == 0:
+        return dx
+    L = lib()
+    aligned = f % 4 == 0 and ldg % 4 == 0 and _al16(g) and _al16(arg)
+    if algo is None:
+        algo = "sell" if aligned and n + csc.num_slots >= 1 << 14 else "row"
+    if algo == "sell":
+        if not aligned:
+            raise ValueError("spmm_max_bwd: the sliced-ELL kernel needs f % 4 == 0 and 16-byte aligned rows")
+        sl = sell_layout(csc)
+        emap = _sell_edge_map(csc, csc2csr)
+        ws_bytes = int(L.gg_spmm_sell_max_workspace_bytes(sl.partial_rows, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        check(L.gg_spmm_sell_max_bwd_f32(_ptr(sl.chunk_ptr), sl.chunks, _ptr(sl.idx), _ptr(emap), _ptr(sl.weights(w_slot_csc)),
+                                         _ptr(sl.vdst), _ptr(sl.hub_rows), _ptr(sl.hub_pptr), sl.hubs, sl.partial_rows,
+                                         _ptr(g), ldg, _ptr(arg), f, n, f, float(self_scale), _ptr(dx), f, _ptr(ws), ws_bytes,
+                                         _spmm_flags(), _stream()), "gg_spmm_sell_max_bwd_f32")
+    elif algo == "row":
+        check(L.gg_spmm_row_max_bwd_f32(_ptr(csc.rowptr), _ptr(csc.nbr), _ptr(csc2csr), _ptr(w_slot_csc), _ptr(g), ldg,
+                                        _ptr(arg), f, n, f, float(self_scale), _ptr(dx), f, _stream()),
+              "gg_spmm_row_max_bwd_f32")
+    else:
+        raise ValueError(f"spmm_max_bwd: algo={algo!r}")
+    return dx
 
 
 class PeerRows:

@@ -234,6 +234,37 @@ int gg_spmm_sell_f32(const uint32_t* chunk_ptr, int64_t chunks, const int32_t* i
                      const float* r1_s, const float* r1_v, const float* r2_s, const float* r2_v, void* workspace,
                      size_t workspace_bytes, int flags, gg_stream_t stream);
 
+/* Max aggregation (csrc/spmm_max.cu; GraphGym cfg.gnn.agg = 'max'):
+ *   out[i,c] = max_{s in segment i} w[s] * x[nbr[s],c] (0 for an empty segment) + self_scale * x_self[i,c] + bias[c]
+ *   arg[i,c] = the first slot s (strict `>` in slot order) that reaches the maximum; -1 for an empty segment
+ *   dx[j,c]  = sum over the CSC slots t of row j with arg[nbr_csc[t],c] == csr_slot(t) of w_csc[t] * g[nbr_csc[t],c]
+ *              + self_scale * g[j,c]
+ * gg_spmm_sell_max_f32 runs on the CSR's sliced-ELL layout (gg_sell_build; slot_of as built, w_sell re-laid by
+ * gg_sell_permute_f32, flags bits 2 / 3 as in gg_spmm_sell_f32); gg_spmm_sell_max_bwd_f32 on the CSC's, with
+ * `edge_map` = gg_sell_compose_map(slot_of of the CSC layout, csc -> csr slot map).  Both need f % 4 == 0 and 16-byte
+ * aligned rows (GG_ERR_UNSUPPORTED / GG_ERR_INVALID otherwise); widths above 128 run as column tiles of <= 128.
+ * Workspace: gg_spmm_sell_max_workspace_bytes(partial rows of the layout, f).  gg_spmm_row_max_f32 /
+ * gg_spmm_row_max_bwd_f32: plain CSR / CSC (+ csc2csr), one warp per row, any f and alignment.  All four are bitwise
+ * run-to-run deterministic; the sliced-ELL and row forwards give the same bits. */
+size_t gg_spmm_sell_max_workspace_bytes(int64_t partial_rows, int64_t f);
+int gg_spmm_sell_max_f32(const uint32_t* chunk_ptr, int64_t chunks, const int32_t* idx, const int32_t* slot_of,
+                         const float* w_sell, const int32_t* vdst, const int32_t* hub_rows, const int32_t* hub_pptr,
+                         int64_t hubs, int64_t partial_rows, const float* x, int64_t ldx, float* out, int64_t ldo,
+                         int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f, const float* x_self, int64_t ld_self,
+                         float self_scale, const float* bias, void* workspace, size_t workspace_bytes, int flags,
+                         gg_stream_t stream);
+int gg_spmm_sell_max_bwd_f32(const uint32_t* chunk_ptr, int64_t chunks, const int32_t* idx, const int32_t* edge_map,
+                             const float* w_sell, const int32_t* vdst, const int32_t* hub_rows, const int32_t* hub_pptr,
+                             int64_t hubs, int64_t partial_rows, const float* g, int64_t ldg, const int32_t* arg,
+                             int64_t ld_arg, int64_t num_rows, int64_t f, float self_scale, float* dx, int64_t ldd,
+                             void* workspace, size_t workspace_bytes, int flags, gg_stream_t stream);
+int gg_spmm_row_max_f32(const int32_t* rowptr, const int32_t* nbr, const float* w_slot, const float* x, int64_t ldx,
+                        float* out, int64_t ldo, int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
+                        const float* x_self, int64_t ld_self, float self_scale, const float* bias, gg_stream_t stream);
+int gg_spmm_row_max_bwd_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* csc2csr, const float* w_slot,
+                            const float* g, int64_t ldg, const int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
+                            float self_scale, float* dx, int64_t ldd, gg_stream_t stream);
+
 /* bf16-gather variant (the north star's 1e-2 mode): x is stored in bf16 (`x_bf16`: raw bf16 bits, ldx in
  * elements, rows 16-byte aligned), products and sums are fp32, out / x_self / bias are fp32.  Same plan and the
  * same fixed summation order as gg_spmm_mpg_f32; needs f % 8 == 0 and f <= 256.  gg_cast_f32_bf16 converts a
