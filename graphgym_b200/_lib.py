@@ -82,6 +82,17 @@ SIGNATURES = {
                                     c_i64, c_f32, c_ptr, c_ptr]),
     "gg_spmm_row_max_bwd_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_f32,
                                         c_ptr, c_i64, c_ptr]),
+    "gg_max_winner_sddmm_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_int, c_i64, c_ptr,
+                                        c_ptr]),
+    "gg_gat_alpha_heads_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_f32, c_ptr, c_ptr]),
+    "gg_gat_dz_heads_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_f32, c_ptr, c_ptr, c_ptr]),
+    "gg_gat_src_sum_heads_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_ptr, c_ptr]),
+    "gg_spmm_row_max_heads_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_int, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64,
+                                          c_ptr, c_ptr]),
+    "gg_spmm_row_max_heads_bwd_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_int, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64,
+                                              c_ptr, c_i64, c_ptr]),
+    "gg_rows_epilogue_f32": (c_int, [c_ptr, c_i64, c_i64, c_i64, c_ptr, c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                     c_i64, c_ptr]),
     "gg_cast_f32_bf16": (c_int, [c_ptr, c_i64, c_i64, c_i64, c_ptr, c_i64, c_ptr]),
     "gg_spmm_mp_bf16": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64,
                                 c_int, c_ptr, c_i64, c_f32, c_ptr, c_ptr, c_size, c_int, c_ptr]),

@@ -7,7 +7,15 @@ loops: the attention runs on the edge list as given.  -> ``functional.gat_aggreg
 GeneralMulAttConvLayer (attconv.py:115-214): logits (<h_i, h_j> + sum(bias_att)) / sqrt(out_channels); the additive
 constant cancels in the softmax (its gradient is zero, as autograd finds in the reference up to rounding), so the layer is
 scaled dot-product attention with Q = K = V = h.  -> the SDDMM / segment-softmax / SpMM passes of contrib/layer/tfg.py.
-Accelerated for the configuration GraphGym ships as default: ``cfg.gnn.normalize_adj = False``, ``cfg.gnn.agg = 'add'``.
+``cfg.gnn.agg`` picks the reduction over a target's in-edges (the edge list as given, duplicates counted):
+  'add'   the sum above (GraphGym's default).
+  'mean'  the sum divided by the in-degree (0 without in-edges), then + bias -> ``functional.gat_aggregate(agg='mean')``
+          on every path the sum takes (fused sliced-ELL, merge-path, row) / ``spmm(MEAN)`` with the alpha weights.
+  'max'   per column the largest message alpha_ij h_j (0 without in-edges), then + bias; torch_scatter's scatter_max:
+          the gradient goes to the first in-edge in edge order that reaches the maximum, and through it to h_j and to
+          alpha_ij (the softmax, att and the scores).  The weighted max of csrc/spmm_max.cu (sliced ELL for heads = 1,
+          a warp-per-row kernel with one weight per (edge, head) otherwise) and the winner SDDMM of csrc/attn_agg.cu.
+``cfg.gnn.normalize_adj = True`` is not on the accelerated path.
 """
 import math
 
@@ -25,14 +33,15 @@ from graphgym_b200.register import register_layer
 
 
 def _check_cfg(name):
-    if cfg.gnn.normalize_adj or cfg.gnn.agg != 'add':
-        raise NotImplementedError(f"{name}: cfg.gnn.normalize_adj / agg != 'add' are not on the accelerated path")
+    if cfg.gnn.normalize_adj or cfg.gnn.agg not in ('add', 'mean', 'max'):
+        raise NotImplementedError(f"{name}: cfg.gnn.normalize_adj / agg {cfg.gnn.agg!r} are not on the accelerated path")
+    return cfg.gnn.agg
 
 
 class GeneralAddAttConvLayer(nn.Module):
     def __init__(self, in_channels, out_channels, improved=False, cached=False, bias=True, **kwargs):
         super().__init__()
-        _check_cfg('gaddconv')
+        self.agg = _check_cfg('gaddconv')
         self.heads = int(cfg.gnn.get('att_heads', 1))
         self.in_channels = in_channels // self.heads * self.heads
         self.out_channels = out_channels // self.heads * self.heads
@@ -55,7 +64,7 @@ class GeneralAddAttConvLayer(nn.Module):
             raise NotImplementedError('edge_weight is never passed by GeneralAddAttConv')
         h = F_.linear(x, self.linear_msg.weight, None)
         layout = get_layout(edge_index, x.size(0), ops.LOOPS_KEEP)
-        return F_.gat_aggregate(h, self.att, self.bias, layout, self.heads, self.negative_slope)
+        return F_.gat_aggregate(h, self.att, self.bias, layout, self.heads, self.negative_slope, self.agg)
 
     def __repr__(self):
         return '{}({}, {}, {})'.format(self.__class__.__name__, self.in_channels, self.out_channels, self.heads)
@@ -64,7 +73,7 @@ class GeneralAddAttConvLayer(nn.Module):
 class GeneralMulAttConvLayer(nn.Module):
     def __init__(self, in_channels, out_channels, improved=False, cached=False, bias=True, **kwargs):
         super().__init__()
-        _check_cfg('gmulconv')
+        self.agg = _check_cfg('gmulconv')
         if int(cfg.gnn.get('att_heads', 1)) != 1:
             raise NotImplementedError('gmulconv: "currently only for single head attention" (attconv.py:134)')
         self.in_channels, self.out_channels = in_channels, out_channels
@@ -81,7 +90,9 @@ class GeneralMulAttConvLayer(nn.Module):
         h = F_.linear(x, self.linear_msg.weight, None)
         layout = get_layout(edge_index, x.size(0), ops.LOOPS_KEEP)
         # 1 / scaler = 1 / sqrt(out_channels); _DotAttention scales by 1 / sqrt(q.size(1)) = the same
-        return _DotAttention.apply(h, h, h, self.bias, layout)
+        if self.agg == 'add':
+            return _DotAttention.apply(h, h, h, self.bias, layout)
+        return F_.dot_attention_aggregate(h, self.bias, layout, self.agg)
 
     def __repr__(self):
         return '{}({}, {}, 1)'.format(self.__class__.__name__, self.in_channels, self.out_channels)

@@ -5,6 +5,8 @@ forward AND backward are ``gg_*`` kernels (no torch math on the path).
   seg_linear   multi-segment dense transform with ID weights  (SURVEY §8a row 9)
   gather_rows / scatter_add_rows   the M-row ID branch of GIN-ID (ref: idconv.py:372-375)
 """
+import math
+
 import torch
 
 from . import ops
@@ -244,8 +246,135 @@ class _GatAggregate(torch.autograd.Function):
         return dh, datt.view_as(att), gb, None, None, None
 
 
-def gat_aggregate(h, att, bias, layout, heads=1, slope=0.2):
+class _GatAggregateMean(torch.autograd.Function):
+    """out[i] = (sum_{j->i} alpha_ij h_j) / indeg(i) + bias: ``_GatAggregate``'s forward without the bias, then the row
+    scale.  Its backward is the sum's backward on g / indeg, with the unscaled sum (kept from the forward, [n, f]) in
+    place of out - bias."""
+
+    @staticmethod
+    def forward(ctx, h, att, bias, layout, heads, slope):
+        h = h.contiguous()
+        need_grad = any(ctx.needs_input_grad[:3])
+        out_sum, alpha, a_tgt, a_src, pos = ops.gat_forward(layout.csr, h, att, heads, slope, None, need_grad)
+        out = ops.rows_epilogue(out_sum, layout.csr, bias=bias)
+        ctx.layout, ctx.heads, ctx.slope, ctx.has_bias = layout, heads, slope, bias is not None
+        ctx.save_for_backward(h, att, alpha, a_tgt, a_src, out_sum, *(pos or ()))
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        h, att, alpha, a_tgt, a_src, out_sum, *pos = ctx.saved_tensors
+        g = g.contiguous()
+        lay = ctx.layout
+        g_mean = ops.rows_epilogue(g, lay.csr)
+        dh, datt = ops.gat_backward(lay.csr, lay.csc, lay.csc2csr, h, att, ctx.heads, ctx.slope, None, alpha, a_tgt, a_src,
+                                    out_sum, g_mean, tuple(pos) or None)
+        gb = ops.colsum(g) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
+        return dh, datt.view_as(att), gb, None, None, None
+
+
+class _GatAggregateMax(torch.autograd.Function):
+    """out[i, c] = max_{j->i} alpha_ij[head(c)] h_j[c] (0 without in-edges) + bias, alpha the GAT attention; the gradient
+    of the max goes to the first in-edge that reaches it, per column, and reaches h_j (scale alpha) and alpha (then the
+    logits, att and h through the scores)."""
+
+    @staticmethod
+    def forward(ctx, h, att, bias, layout, heads, slope):
+        h = h.contiguous()
+        csr = layout.csr
+        if heads == 1:
+            a_tgt, a_src = ops.gat_scores(h, att.view(1, -1))
+            alpha = ops.gat_alpha(csr, a_tgt, a_src, slope)
+            out, arg = ops.spmm_max(csr, h, alpha, bias=bias)
+        else:
+            a_tgt, a_src = ops.gat_scores_heads(h, att, heads)
+            alpha = ops.gat_alpha_heads(csr, a_tgt, a_src, heads, slope)
+            out, arg = ops.spmm_max_heads(csr, h, alpha, heads, bias)
+        ctx.layout, ctx.heads, ctx.slope, ctx.has_bias = layout, heads, slope, bias is not None
+        ctx.save_for_backward(h, att, a_tgt, a_src, alpha, arg)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        h, att, a_tgt, a_src, alpha, arg = ctx.saved_tensors
+        g = g.contiguous()
+        lay, heads, slope = ctx.layout, ctx.heads, ctx.slope
+        csr, csc, m = lay.csr, lay.csc, lay.csc2csr
+        c = h.size(1) // heads
+        att2 = att.view(heads, 2 * c)
+        att_tgt, att_src = att2[:, :c].contiguous().view(-1), att2[:, c:].contiguous().view(-1)
+        dalpha = ops.max_winner_sddmm(csr, arg, g, h, heads)
+        if heads == 1:
+            dz, da_tgt = ops.gat_dz(csr, a_tgt, a_src, alpha, dalpha.view(-1), slope)
+            alpha_t, da_src = ops.gat_csc_gather(csc, m, alpha, dz)
+            dh = ops.spmm_max_bwd(csc, m, g, arg, alpha_t)
+        else:
+            dz, da_tgt = ops.gat_dz_heads(csr, a_tgt, a_src, alpha, dalpha, heads, slope)
+            da_src = ops.gat_src_sum_heads(csc, m, dz, heads)
+            dh = ops.spmm_max_heads_bwd(csc, m, g, arg, alpha, heads)
+        # + da_src att_src + da_tgt att_tgt: the scores a_src = att_src . h, a_tgt = att_tgt . h
+        ops.rows_epilogue(dh, rank1=(da_src, att_src, da_tgt, att_tgt), heads=heads, out=dh)
+        datt = ops.gat_att_grad(h, da_tgt, da_src, heads)
+        gb = ops.colsum(g) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
+        return dh, datt.view_as(att), gb, None, None, None
+
+
+def gat_aggregate(h, att, bias, layout, heads=1, slope=0.2, agg="add"):
+    """``agg``: 'add' (sum over the in-edges), 'mean' or 'max'."""
+    if agg == "mean":
+        return _GatAggregateMean.apply(h, att, bias, layout, int(heads), float(slope))
+    if agg == "max":
+        return _GatAggregateMax.apply(h, att, bias, layout, int(heads), float(slope))
     return _GatAggregate.apply(h, att, bias, layout, int(heads), float(slope))
+
+
+class _DotAttentionAgg(torch.autograd.Function):
+    """out[i] = mean or max over j->i of softmax_i(<h_i, h_j> / sqrt(f)) h_j (+ bias): gmulconv's Q = K = V = h with a
+    mean or max instead of the sum.  The backward sums the three gradient terms through the epilogues of the SpMMs."""
+
+    @staticmethod
+    def forward(ctx, h, bias, layout, agg):
+        h = h.contiguous()
+        csr = layout.csr
+        scale = 1.0 / math.sqrt(h.size(1))
+        z = ops.sddmm(csr, h, h)
+        alpha = ops.segment_softmax(csr, z, scale)
+        arg = None
+        if agg == "max":
+            out, arg = ops.spmm_max(csr, h, alpha, bias=bias)
+        else:
+            out = ops.spmm(csr, h, alpha, ops.MEAN, None, 0.0, bias)
+        ctx.layout, ctx.scale, ctx.agg, ctx.has_bias = layout, scale, agg, bias is not None
+        ctx.save_for_backward(h, alpha, arg)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        h, alpha, arg = ctx.saved_tensors
+        lay = ctx.layout
+        csr, csc, m = lay.csr, lay.csc, lay.csc2csr
+        g = g.contiguous()
+        if ctx.agg == "max":
+            dalpha = ops.max_winner_sddmm(csr, arg, g, h).view(-1)
+        else:
+            g_mean = ops.rows_epilogue(g, csr)
+            dalpha = ops.sddmm(csr, h, g_mean)
+        dz = ops.segment_softmax_bwd(csr, alpha, dalpha, ctx.scale)
+        alpha_t, _ = ops.gat_csc_gather(csc, m, alpha, dz)
+        dz_t, _ = ops.gat_csc_gather(csc, m, dz, dz)
+        if ctx.agg == "max":
+            dv = ops.spmm_max_bwd(csc, m, g, arg, alpha_t)
+        else:
+            dv = ops.spmm(csc, g_mean, alpha_t)
+        dq = ops.spmm(csr, h, dz, ops.SUM, dv, 1.0)          # + dv in the epilogue
+        dh = ops.spmm(csc, h, dz_t, ops.SUM, dq, 1.0)        # dk + dq + dv
+        gb = ops.colsum(g) if (ctx.has_bias and ctx.needs_input_grad[1]) else None
+        return dh, gb, None, None
+
+
+def dot_attention_aggregate(h, bias, layout, agg):
+    """gmulconv's attention with ``agg`` in ('mean', 'max'); 'add' is ``tfg._DotAttention``."""
+    return _DotAttentionAgg.apply(h, bias, layout, agg)
 
 
 class _PostOps(torch.autograd.Function):

@@ -420,6 +420,69 @@ def spmm_max_bwd(csc, csc2csr, g, arg, w_slot_csc=None, self_scale=0.0, algo=Non
     return dx
 
 
+def spmm_max_heads(csr, x, w, heads, bias=None):
+    """``spmm_max`` with one weight per (slot, head): column c of x uses w[s, c // (f / heads)] (w [E', heads]); the
+    warp-per-row kernel (csrc/attn_agg.cu).  -> (out [n, f], arg int32 [n, f])."""
+    _need_cuda(x, w, bias, csr.rowptr)
+    x, ldx = _rows(x, "x")
+    n, f = csr.num_nodes, x.size(1)
+    out = torch.empty((n, f), dtype=torch.float32, device=x.device)
+    arg = torch.empty((n, f), dtype=torch.int32, device=x.device)
+    if bias is not None:
+        bias = bias.contiguous()
+    check(lib().gg_spmm_row_max_heads_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(w.contiguous()), int(heads), _ptr(x), ldx,
+                                          _ptr(out), f, _ptr(arg), f, n, f, _ptr(bias), _stream()),
+          "gg_spmm_row_max_heads_f32")
+    return out, arg
+
+
+def spmm_max_heads_bwd(csc, csc2csr, g, arg, w, heads):
+    """Backward of ``spmm_max_heads`` wrt x; ``w`` in CSR slot order [E', heads]."""
+    _need_cuda(g, arg, w, csc.rowptr)
+    g, ldg = _rows(g, "g")
+    arg = arg.contiguous()
+    n, f = csc.num_nodes, g.size(1)
+    dx = torch.empty((n, f), dtype=torch.float32, device=g.device)
+    check(lib().gg_spmm_row_max_heads_bwd_f32(_ptr(csc.rowptr), _ptr(csc.nbr), _ptr(csc2csr), _ptr(w.contiguous()),
+                                              int(heads), _ptr(g), ldg, _ptr(arg), f, n, f, _ptr(dx), f, _stream()),
+          "gg_spmm_row_max_heads_bwd_f32")
+    return dx
+
+
+def max_winner_sddmm(csr, arg, g, h, heads=1):
+    """dalpha [E', heads]: dalpha[s, k] = sum over the columns c of head k that slot s won (arg[i, c] == s) of
+    g[i, c] * h[nbr[s], c] — the gradient of per-slot weights through ``spmm_max`` / ``spmm_max_heads``; bitwise
+    deterministic (csrc/attn_agg.cu)."""
+    _need_cuda(g, h, arg, csr.rowptr)
+    g, ldg = _rows(g, "g")
+    h, ldh = _rows(h, "h")
+    arg = arg.contiguous()
+    f = g.size(1)
+    dalpha = _f32((csr.num_slots, heads), g.device)
+    check(lib().gg_max_winner_sddmm_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(arg), f, _ptr(g), ldg, _ptr(h), ldh,
+                                        csr.num_nodes, int(heads), f, _ptr(dalpha), _stream()), "gg_max_winner_sddmm_f32")
+    return dalpha
+
+
+def rows_epilogue(x, mean_csr=None, rank1=None, heads=1, bias=None, out=None):
+    """out[i, :] = x[i, :] / indeg(i) (with ``mean_csr``; rows without in-edges unscaled) + s1[i, k] v1 + s2[i, k] v2
+    (``rank1`` = (s1 [n, heads], v1 [f], s2, v2), k the column's head) + bias.  ``out`` may be ``x``."""
+    _need_cuda(x, bias)
+    x, ldx = _rows(x, "x")
+    n, f = x.shape
+    if out is None:
+        out = torch.empty((n, f), dtype=torch.float32, device=x.device)
+    out_t, ldo = _rows(out, "out")
+    assert out_t is out, "out must have unit inner stride"
+    r1 = [t.contiguous() if t is not None else None for t in (rank1 or (None, None, None, None))]
+    if bias is not None:
+        bias = bias.contiguous()
+    check(lib().gg_rows_epilogue_f32(_ptr(x), ldx, n, f, _ptr(mean_csr.rowptr if mean_csr is not None else None),
+                                     int(heads), _ptr(r1[0]), _ptr(r1[1]), _ptr(r1[2]), _ptr(r1[3]), _ptr(bias), _ptr(out),
+                                     ldo, _stream()), "gg_rows_epilogue_f32")
+    return out
+
+
 class PeerRows:
     """Where the rows of a peer-output SpMM go: ``ptrs[o]`` = device pointer (peer memory, already offset
     to this rank's column slice) of rank o's [rows_per_rank, ld] block."""
@@ -984,14 +1047,53 @@ def gat_csc_gather(csc, csc2csr, alpha, dz):
     return alpha_t, da_src
 
 
-def gat_att_grad(h, da_tgt, da_src):
-    """datt [1, 2c] = [da_tgt^T h | da_src^T h] over the rows of ``h``."""
+def gat_att_grad(h, da_tgt, da_src, heads=1):
+    """datt [heads, 2c] = per head [da_tgt^T h | da_src^T h] over the rows of ``h`` (da_* [n, heads])."""
     h, ldh = _rows(h, "h")
-    n, c = h.shape
+    n, f = h.shape
+    c = f // heads
     L = lib()
-    datt = torch.empty((1, 2 * c), dtype=torch.float32, device=h.device)
-    ws_bytes = int(L.gg_gat_att_grad_workspace_bytes(n, 1, c))
+    datt = torch.empty((heads, 2 * c), dtype=torch.float32, device=h.device)
+    ws_bytes = int(L.gg_gat_att_grad_workspace_bytes(n, heads, c))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=h.device)
-    check(L.gg_gat_att_grad_f32(_ptr(h), ldh, _ptr(da_tgt.contiguous()), _ptr(da_src.contiguous()), n, 1, c, _ptr(datt),
+    check(L.gg_gat_att_grad_f32(_ptr(h), ldh, _ptr(da_tgt.contiguous()), _ptr(da_src.contiguous()), n, heads, c, _ptr(datt),
                                 _ptr(ws), ws_bytes, _stream()), "gg_gat_att_grad_f32")
     return datt
+
+
+# ---- per-(slot, head) passes of the multi-head max (csrc/attn_agg.cu) -----------------------------------
+def gat_scores_heads(h, att, heads):
+    """-> a_tgt, a_src [n, heads] of ``gat_forward`` (``att`` [1, heads, 2c])."""
+    _need_cuda(h, att)
+    h, ldh = _rows(h, "h")
+    n, f = h.shape
+    a_tgt, a_src = _f32((n, heads), h.device), _f32((n, heads), h.device)
+    check(lib().gg_gat_scores_f32(_ptr(h), ldh, _ptr(att.contiguous()), n, heads, f // heads, _ptr(a_tgt), _ptr(a_src),
+                                  _stream()), "gg_gat_scores_f32")
+    return a_tgt, a_src
+
+
+def gat_alpha_heads(csr, a_tgt, a_src, heads, slope):
+    alpha = _f32((csr.num_slots, heads), a_tgt.device)
+    check(lib().gg_gat_alpha_heads_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(a_tgt.contiguous()), _ptr(a_src.contiguous()),
+                                       csr.num_nodes, int(heads), float(slope), _ptr(alpha), _stream()),
+          "gg_gat_alpha_heads_f32")
+    return alpha
+
+
+def gat_dz_heads(csr, a_tgt, a_src, alpha, dalpha, heads, slope):
+    """-> dz [E', heads], da_tgt [n, heads]."""
+    dev = alpha.device
+    dz, da_tgt = _f32((csr.num_slots, heads), dev), _f32((csr.num_nodes, heads), dev)
+    check(lib().gg_gat_dz_heads_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(a_tgt), _ptr(a_src), _ptr(alpha),
+                                    _ptr(dalpha.contiguous()), csr.num_nodes, int(heads), float(slope), _ptr(dz),
+                                    _ptr(da_tgt), _stream()), "gg_gat_dz_heads_f32")
+    return dz, da_tgt
+
+
+def gat_src_sum_heads(csc, csc2csr, dz, heads):
+    """-> da_src [n, heads] = per-source sums of dz."""
+    da_src = _f32((csc.num_nodes, heads), dz.device)
+    check(lib().gg_gat_src_sum_heads_f32(_ptr(csc.rowptr), _ptr(csc2csr), _ptr(dz), csc.num_nodes, int(heads),
+                                         _ptr(da_src), _stream()), "gg_gat_src_sum_heads_f32")
+    return da_src

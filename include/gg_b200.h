@@ -265,6 +265,40 @@ int gg_spmm_row_max_bwd_f32(const int32_t* rowptr, const int32_t* nbr, const int
                             const float* g, int64_t ldg, const int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
                             float self_scale, float* dx, int64_t ldd, gg_stream_t stream);
 
+/* Mean / max aggregation of the attention layers (csrc/attn_agg.cu; gaddconv / gmulconv with cfg.gnn.agg = 'mean' /
+ * 'max').  heads H splits f into H blocks of c = f / H columns; column col belongs to head col / c.
+ *   gg_max_winner_sddmm_f32   dalpha[s*H + k] = sum over the columns col of head k with arg[i,col] == s (s a slot of CSR
+ *                             row i) of g[i,col] * h[nbr[s],col]; 0 for a slot that won nothing.  The gradient of the
+ *                             attention weights through the max; bitwise run-to-run deterministic (column order).
+ *   gg_gat_alpha_heads_f32    alpha[s*H + k] = softmax over row i of leaky_relu(a_tgt[i*H+k] + a_src[nbr[s]*H+k])
+ *                             (max-shifted, denominator + 1e-16), as gg_gat_alpha_f32 per head
+ *   gg_gat_dz_heads_f32       gg_gat_dz_f32 per head: dz[s*H+k], da_tgt[i*H+k]
+ *   gg_gat_src_sum_heads_f32  da_src[j*H+k] = sum over the CSC slots t of row j of dz[slot_map[t]*H + k]
+ *   gg_spmm_row_max_heads_f32 gg_spmm_row_max_f32 with weight w[s*H + col/c] (+ bias), one warp per row
+ *   gg_spmm_row_max_heads_bwd_f32  its backward on the CSC layout: w indexed by the CSR slot csc2csr[t]
+ *   gg_rows_epilogue_f32      out[i,col] = x[i,col] * (1/indeg(i) if rowptr, indeg = rowptr[i+1] - rowptr[i], rows
+ *                             without slots unscaled) + s1[i*H+k] v1[col] + s2[i*H+k] v2[col] (if s1) + bias[col];
+ *                             element-wise, out may alias x. */
+int gg_max_winner_sddmm_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* arg, int64_t ld_arg, const float* g,
+                            int64_t ldg, const float* h, int64_t ldh, int64_t num_rows, int heads, int64_t f, float* dalpha,
+                            gg_stream_t stream);
+int gg_gat_alpha_heads_f32(const int32_t* rowptr, const int32_t* nbr, const float* a_tgt, const float* a_src,
+                           int64_t num_rows, int heads, float slope, float* alpha, gg_stream_t stream);
+int gg_gat_dz_heads_f32(const int32_t* rowptr, const int32_t* nbr, const float* a_tgt, const float* a_src,
+                        const float* alpha, const float* dalpha, int64_t num_rows, int heads, float slope, float* dz,
+                        float* da_tgt, gg_stream_t stream);
+int gg_gat_src_sum_heads_f32(const int32_t* rowptr_t, const int32_t* slot_map, const float* dz, int64_t num_rows,
+                             int heads, float* da_src, gg_stream_t stream);
+int gg_spmm_row_max_heads_f32(const int32_t* rowptr, const int32_t* nbr, const float* w, int heads, const float* x,
+                              int64_t ldx, float* out, int64_t ldo, int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
+                              const float* bias, gg_stream_t stream);
+int gg_spmm_row_max_heads_bwd_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* csc2csr, const float* w,
+                                  int heads, const float* g, int64_t ldg, const int32_t* arg, int64_t ld_arg, int64_t num_rows,
+                                  int64_t f, float* dx, int64_t ldd, gg_stream_t stream);
+int gg_rows_epilogue_f32(const float* x, int64_t ldx, int64_t num_rows, int64_t f, const int32_t* rowptr, int heads,
+                         const float* s1, const float* v1, const float* s2, const float* v2, const float* bias, float* out,
+                         int64_t ldo, gg_stream_t stream);
+
 /* bf16-gather variant (the north star's 1e-2 mode): x is stored in bf16 (`x_bf16`: raw bf16 bits, ldx in
  * elements, rows 16-byte aligned), products and sums are fp32, out / x_self / bias are fp32.  Same plan and the
  * same fixed summation order as gg_spmm_mpg_f32; needs f % 8 == 0 and f <= 256.  gg_cast_f32_bf16 converts a
