@@ -168,6 +168,11 @@ SIGNATURES = {
                                    c_i64, c_ptr, c_ptr]),
     "gg_postops_bwd_f32": (c_int, [c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_ptr, c_ptr, c_ptr, c_int,
                                    c_int, c_f32, c_int, c_ptr, c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_size, c_ptr]),
+    "gg_postops_skip_fwd_f32": (c_int, [c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_i64, c_int, c_ptr, c_ptr, c_ptr,
+                                        c_ptr, c_int, c_f32, c_int, c_ptr, c_i64, c_ptr, c_ptr]),
+    "gg_postops_skip_bwd_f32": (c_int, [c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_i64, c_int, c_ptr,
+                                        c_ptr, c_ptr, c_int, c_int, c_f32, c_int, c_ptr, c_ptr, c_i64, c_ptr, c_i64,
+                                        c_ptr, c_ptr, c_ptr, c_size, c_ptr]),
     "gg_segment_softmax_f32": (c_int, [c_ptr, c_ptr, c_i64, c_f32, c_ptr, c_ptr]),
     "gg_segment_softmax_bwd_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_f32, c_ptr, c_ptr]),
     "gg_gat_sell_workspace_bytes": (c_size, [c_i64, c_i64]),

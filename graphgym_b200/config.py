@@ -22,7 +22,8 @@ def _defaults():
     c = _Node()
     c.gnn = _Node(layers_pre_mp=0, layers_mp=2, layers_post_mp=0, dim_inner=16, layer_type='generalconv',
                   stage_type='stack', batchnorm=True, act='relu', dropout=0.0, agg='add',
-                  normalize_adj=False, l2norm=True, keep_edge=0.5, self_msg='concat', att_heads=1)
+                  normalize_adj=False, l2norm=True, keep_edge=0.5, self_msg='concat', att_heads=1,
+                  skip_every=1)
     c.bn = _Node(eps=1e-5, mom=0.1)
     c.mem = _Node(inplace=False)
     c.dataset = _Node(transform='none', augment_feature=[], augment_feature_dims=[])

@@ -11,6 +11,13 @@
 // where dA (gradient at the pre-activation) is recomputed per row from the saved OUTPUT: the activation's gate is the
 // sign of the output (ReLU / leaky ReLU, slope > 0), the L2 backward needs <go, out> per row and the saved row norm.
 // No atomics: every column reduction is per-CTA partials + a fixed-order merge => deterministic.
+//
+// The skip blocks of GNNSkipStage (ref: graphgym/models/gnn.py GNNSkipBlock) end in "BN, + the block input (or
+// concatenate it), activation"; the same kernels take that residual operand (gg_postops_skip_*_f32, res_mode):
+//   SUM     out = l2?(act(BN(y) + res))                             res [n, f]
+//   PREFIX  out = l2?([act(res) | act(BN(y))])                      res [n, p], out [n, p + f], the L2 over all p + f
+// The backward writes dres = dA beside dy (SUM: the f columns; PREFIX: the p prefix columns) and dy = BN-backward(dA);
+// the L2 row dot covers the whole output row, the dgamma / dbeta column sums the f columns only.
 #include "common.cuh"
 
 namespace gg {
@@ -41,6 +48,12 @@ struct PostArgs {
     const float* dgamma;  // backward apply (train): column sums from the reduce pass
     const float* dbeta;
     float* partial;       // reduce pass: [grid, 2, f]
+    int res_mode;         // GG_SKIP_NONE / GG_SKIP_SUM / GG_SKIP_PREFIX
+    const float* res;     // forward: the skip operand [n, ld_res] (SUM: f columns, PREFIX: p columns)
+    int64_t ld_res;
+    int p;                // PREFIX: width of the carried columns; the f columns of out and go start at column p (else 0)
+    float* dres;          // backward apply: gradient wrt res [n, ld_dres]
+    int64_t ld_dres;
 };
 
 __device__ __forceinline__ float po_act(float a, int act, float slope) {
@@ -52,6 +65,20 @@ __device__ __forceinline__ float po_act_grad(float o, int act, float slope) {  /
     if (act == GG_ACT_RELU) return o > 0.f ? 1.f : 0.f;
     if (act == GG_ACT_LRELU) return o > 0.f ? 1.f : slope;
     return 1.f;
+}
+template <int V>
+__device__ __forceinline__ void po_ld(float (&v)[V], const float* p) {
+    if constexpr (V == 4) {
+        const float4 t = *reinterpret_cast<const float4*>(p);
+        v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+    } else {
+        v[0] = *p;
+    }
+}
+template <int V>
+__device__ __forceinline__ void po_st(float* p, const float (&v)[V]) {
+    if constexpr (V == 4) *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
+    else *p = v[0];
 }
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
@@ -178,22 +205,37 @@ __global__ void __launch_bounds__(kPoThreads) postops_fwd_kernel(const __grid_co
     constexpr int kKeep = 4;   // column groups of a row a lane keeps in registers (f <= 512 with V = 4)
     for (int64_t r = (int64_t)blockIdx.x * kPoWarps + (threadIdx.x >> 5); r < a.n; r += warps) {
         const float* yr = a.y + r * a.ld_y;
-        float* orow = a.dst + r * a.ld_dst;
+        const float* rr = a.res + r * a.ld_res;       // only read when res_mode != NONE
+        float* prow = a.dst + r * a.ld_dst;           // PREFIX: act(res) in [0, p)
+        float* orow = prow + a.p;
         float keep[kKeep][V];
         float ss = 0.f;
+        if (a.res_mode == GG_SKIP_PREFIX) {
+            for (int c = lane * V; c < a.p; c += 32 * V) {
+                float v[V];
+                po_ld<V>(v, rr + c);
+#pragma unroll
+                for (int q = 0; q < V; ++q) {
+                    v[q] = po_act(v[q], a.act, a.slope);
+                    ss = fmaf(v[q], v[q], ss);
+                }
+                if (!a.l2) po_st<V>(prow + c, v);
+            }
+        }
         int k = 0;
         for (int c = lane * V; c < a.f; c += 32 * V, ++k) {
-            float v[V];
-            if (V == 4) *reinterpret_cast<float4*>(v) = *reinterpret_cast<const float4*>(yr + c);
-            else v[0] = yr[c];
+            float v[V], s[V];
+#pragma unroll
+            for (int q = 0; q < V; ++q) s[q] = -0.f;   // x + (-0) == x bitwise: no residual leaves the result as it was
+            po_ld<V>(v, yr + c);
+            if (a.res_mode == GG_SKIP_SUM) po_ld<V>(s, rr + c);
 #pragma unroll
             for (int q = 0; q < V; ++q) {
-                v[q] = po_act(fmaf(v[q] - pc.mu[c + q], pc.isg[c + q], pc.beta[c + q]), a.act, a.slope);
+                v[q] = po_act(fmaf(v[q] - pc.mu[c + q], pc.isg[c + q], pc.beta[c + q]) + s[q], a.act, a.slope);
                 ss = fmaf(v[q], v[q], ss);
             }
             if (!a.l2) {
-                if (V == 4) *reinterpret_cast<float4*>(orow + c) = *reinterpret_cast<float4*>(v);
-                else orow[c] = v[0];
+                po_st<V>(orow + c, v);
             } else if (k < kKeep) {
 #pragma unroll
                 for (int q = 0; q < V; ++q) keep[k][q] = v[q];
@@ -203,6 +245,15 @@ __global__ void __launch_bounds__(kPoThreads) postops_fwd_kernel(const __grid_co
         const float nrm = fmaxf(sqrtf(warp_sum(ss)), 1e-12f);   // F.normalize: x / max(||x||, eps)
         if (lane == 0) a.rownorm[r] = nrm;
         const float scale = 1.f / nrm;
+        if (a.res_mode == GG_SKIP_PREFIX) {   // the carried columns are recomputed from the (L1-resident) res row
+            for (int c = lane * V; c < a.p; c += 32 * V) {
+                float v[V];
+                po_ld<V>(v, rr + c);
+#pragma unroll
+                for (int q = 0; q < V; ++q) v[q] = po_act(v[q], a.act, a.slope) * scale;
+                po_st<V>(prow + c, v);
+            }
+        }
         k = 0;
         for (int c = lane * V; c < a.f; c += 32 * V, ++k) {
             float v[V];
@@ -210,27 +261,32 @@ __global__ void __launch_bounds__(kPoThreads) postops_fwd_kernel(const __grid_co
 #pragma unroll
                 for (int q = 0; q < V; ++q) v[q] = keep[k][q] * scale;
             } else {   // very wide rows: recompute from the (L1-resident) row
-                if (V == 4) *reinterpret_cast<float4*>(v) = *reinterpret_cast<const float4*>(yr + c);
-                else v[0] = yr[c];
+                float s[V];
+#pragma unroll
+                for (int q = 0; q < V; ++q) s[q] = -0.f;
+                po_ld<V>(v, yr + c);
+                if (a.res_mode == GG_SKIP_SUM) po_ld<V>(s, rr + c);
 #pragma unroll
                 for (int q = 0; q < V; ++q)
-                    v[q] = po_act(fmaf(v[q] - pc.mu[c + q], pc.isg[c + q], pc.beta[c + q]), a.act, a.slope) * scale;
+                    v[q] = po_act(fmaf(v[q] - pc.mu[c + q], pc.isg[c + q], pc.beta[c + q]) + s[q], a.act, a.slope) *
+                           scale;
             }
-            if (V == 4) *reinterpret_cast<float4*>(orow + c) = *reinterpret_cast<float4*>(v);
-            else orow[c] = v[0];
+            po_st<V>(orow + c, v);
         }
     }
 }
 
 // ---- backward ------------------------------------------------------------------------------------------------------
-// dA for the columns of one row a lane owns: L2 backward (needs the row's <go, out>), then the activation's gate
+// dA for the columns of one row a lane owns: L2 backward (needs the row's <go, out>, over the whole row: PREFIX columns
+// included), then the activation's gate
 template <int V>
 __device__ __forceinline__ float po_row_dot(const PostArgs& a, int64_t r, int lane) {
     if (!a.l2) return 0.f;
     const float* gr = a.go + r * a.ld_go;
     const float* orow = a.out + r * a.ld_o;
+    const int w = a.p + a.f;
     float d = 0.f;
-    for (int c = lane * V; c < a.f; c += 32 * V) {
+    for (int c = lane * V; c < w; c += 32 * V) {
         if (V == 4) {
             const float4 g = *reinterpret_cast<const float4*>(gr + c), o = *reinterpret_cast<const float4*>(orow + c);
             d = fmaf(g.x, o.x, fmaf(g.y, o.y, fmaf(g.z, o.z, fmaf(g.w, o.w, d))));
@@ -261,8 +317,8 @@ __global__ void __launch_bounds__(kPoThreads) postops_bwd_reduce_kernel(const __
     for (int64_t r = r0 + wid; r < r1; r += kPoWarps) {
         const float dot = po_row_dot<V>(a, r, lane);
         const float inv_norm = a.l2 ? 1.f / a.rownorm[r] : 1.f;
-        const float* gr = a.go + r * a.ld_go;
-        const float* orow = a.out + r * a.ld_o;
+        const float* gr = a.go + r * a.ld_go + a.p;   // the f columns only (PREFIX: after the carried ones)
+        const float* orow = a.out + r * a.ld_o + a.p;
         const float* yr = a.y + r * a.ld_y;
         for (int c = lane * V; c < a.f; c += 32 * V) {
             float g[V], o[V], yv[V];
@@ -329,12 +385,13 @@ __global__ void __launch_bounds__(kPoThreads) postops_bwd_apply_kernel(const __g
     for (int64_t r = (int64_t)blockIdx.x * kPoWarps + (threadIdx.x >> 5); r < a.n; r += warps) {
         const float dot = po_row_dot<V>(a, r, lane);
         const float inv_norm = a.l2 ? 1.f / a.rownorm[r] : 1.f;
-        const float* gr = a.go + r * a.ld_go;
-        const float* orow = a.out + r * a.ld_o;
+        const float* gr = a.go + r * a.ld_go + a.p;   // the f columns (PREFIX: after the carried ones)
+        const float* orow = a.out + r * a.ld_o + a.p;
         const float* yr = a.y + r * a.ld_y;
         float* drow = a.dst + r * a.ld_dst;
+        float* rrow = a.dres + r * a.ld_dres;         // only written when res_mode != NONE
         for (int c = lane * V; c < a.f; c += 32 * V) {
-            float g[V], o[V], yv[V];
+            float g[V], o[V], yv[V], da[V];
             if (V == 4) {
                 *reinterpret_cast<float4*>(g) = *reinterpret_cast<const float4*>(gr + c);
                 *reinterpret_cast<float4*>(o) = *reinterpret_cast<const float4*>(orow + c);
@@ -346,6 +403,7 @@ __global__ void __launch_bounds__(kPoThreads) postops_bwd_apply_kernel(const __g
 #pragma unroll
             for (int q = 0; q < V; ++q) {
                 float d = po_da(a, g[q], o[q], dot, inv_norm);
+                da[q] = d;                                // dA (SUM: dres)
                 if (a.mean) {
                     if (a.train) {
                         const float xhat = (yv[q] - s_mu[c + q]) * s_is[c + q];
@@ -357,6 +415,17 @@ __global__ void __launch_bounds__(kPoThreads) postops_bwd_apply_kernel(const __g
             }
             if (V == 4) *reinterpret_cast<float4*>(drow + c) = *reinterpret_cast<float4*>(g);
             else drow[c] = g[0];
+            if (a.res_mode == GG_SKIP_SUM) po_st<V>(rrow + c, da);
+        }
+        if (a.res_mode == GG_SKIP_PREFIX) {           // dres = dA on the carried columns
+            for (int c = lane * V; c < a.p; c += 32 * V) {
+                float g[V], o[V];
+                po_ld<V>(g, gr - a.p + c);
+                po_ld<V>(o, orow - a.p + c);
+#pragma unroll
+                for (int q = 0; q < V; ++q) g[q] = po_da(a, g[q], o[q], dot, inv_norm);
+                po_st<V>(rrow + c, g);
+            }
         }
     }
 }
@@ -424,20 +493,23 @@ static int po_check(const char* who, int64_t n, int64_t f, int act) {
     return GG_OK;
 }
 
-int gg_postops_fwd_f32(const float* y, int64_t ld_y, int64_t n, int64_t f, const float* mean, const float* invstd,
-                       const float* gamma, const float* beta, int act, float slope, int l2norm, float* out,
-                       int64_t ld_out, float* rownorm, gg_stream_t stream) {
-    int rc = po_check("gg_postops_fwd_f32", n, f, act);
+// forward and backward of both the plain post-ops (res_mode NONE) and the skip epilogue
+static int po_fwd(const char* who, const float* y, int64_t ld_y, const float* res, int64_t ld_res, int64_t n, int64_t f,
+                  int64_t p, int mode, const float* mean, const float* invstd, const float* gamma, const float* beta,
+                  int act, float slope, int l2norm, float* out, int64_t ld_out, float* rownorm, gg_stream_t stream) {
+    int rc = po_check(who, n, f, act);
     if (rc != GG_OK) return rc;
     if (n == 0) return GG_OK;
-    GG_REQUIRE(y && out && ld_y >= f && ld_out >= f && (!mean || invstd) && (!gamma || beta) && (!l2norm || rownorm),
-               "gg_postops_fwd_f32: bad operands");
+    GG_REQUIRE(y && out && ld_y >= f && ld_out >= p + f && (!mean || invstd) && (!gamma || beta) && (!l2norm || rownorm),
+               "%s: bad operands", who);
+    GG_REQUIRE(mode == GG_SKIP_NONE || (res && ld_res >= (mode == GG_SKIP_SUM ? f : p)), "%s: bad residual", who);
     PostArgs a{};
     a.y = y; a.ld_y = ld_y; a.dst = out; a.ld_dst = ld_out; a.n = n; a.f = (int)f; a.mean = mean; a.invstd = invstd;
     a.gamma = gamma; a.beta = beta; a.act = act; a.slope = slope; a.l2 = l2norm; a.rownorm = rownorm;
-    const bool vec = f % 4 == 0 && po_vec_ok(y, ld_y) && po_vec_ok(out, ld_out);
+    a.res_mode = mode; a.res = res; a.ld_res = ld_res; a.p = (int)p;
+    const bool vec = f % 4 == 0 && p % 4 == 0 && po_vec_ok(y, ld_y) && po_vec_ok(out, ld_out) && po_vec_ok(res, ld_res);
     const size_t smem = (size_t)3 * f * sizeof(float);
-    GG_REQUIRE(smem <= 200 * 1024, "gg_postops_fwd_f32: f=%lld too wide", (long long)f);
+    GG_REQUIRE(smem <= 200 * 1024, "%s: f=%lld too wide", who, (long long)f);
     if (vec) {
         GG_CUDA(cudaFuncSetAttribute(postops_fwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         postops_fwd_kernel<4><<<po_row_grid(n), kPoThreads, smem, as_stream(stream)>>>(a);
@@ -449,18 +521,21 @@ int gg_postops_fwd_f32(const float* y, int64_t ld_y, int64_t n, int64_t f, const
     return GG_OK;
 }
 
-int gg_postops_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t ld_out, const float* y, int64_t ld_y,
-                       int64_t n, int64_t f, const float* mean, const float* invstd, const float* gamma, int train,
-                       int act, float slope, int l2norm, const float* rownorm, float* dy, int64_t ld_dy, float* dgamma,
-                       float* dbeta, void* workspace, size_t workspace_bytes, gg_stream_t stream) {
-    int rc = po_check("gg_postops_bwd_f32", n, f, act);
+static int po_bwd(const char* who, const float* go, int64_t ld_go, const float* out, int64_t ld_out, const float* y,
+                  int64_t ld_y, int64_t n, int64_t f, int64_t p, int mode, const float* mean, const float* invstd,
+                  const float* gamma, int train, int act, float slope, int l2norm, const float* rownorm, float* dy,
+                  int64_t ld_dy, float* dres, int64_t ld_dres, float* dgamma, float* dbeta, void* workspace,
+                  size_t workspace_bytes, gg_stream_t stream) {
+    int rc = po_check(who, n, f, act);
     if (rc != GG_OK) return rc;
     if (n == 0) return GG_OK;
-    GG_REQUIRE(go && out && dy && ld_go >= f && ld_out >= f && ld_dy >= f && (!mean || (invstd && y && ld_y >= f)) &&
-                   (!l2norm || rownorm) && (!mean || (dgamma && dbeta && workspace)),
-               "gg_postops_bwd_f32: bad operands");
+    GG_REQUIRE(go && out && dy && ld_go >= p + f && ld_out >= p + f && ld_dy >= f &&
+                   (!mean || (invstd && y && ld_y >= f)) && (!l2norm || rownorm) &&
+                   (!mean || (dgamma && dbeta && workspace)),
+               "%s: bad operands", who);
+    GG_REQUIRE(mode == GG_SKIP_NONE || (dres && ld_dres >= (mode == GG_SKIP_SUM ? f : p)), "%s: bad residual", who);
     if (mean && workspace_bytes < gg_postops_workspace_bytes(n, f)) {
-        set_error("gg_postops_bwd_f32: workspace %zu < %zu", workspace_bytes, gg_postops_workspace_bytes(n, f));
+        set_error("%s: workspace %zu < %zu", who, workspace_bytes, gg_postops_workspace_bytes(n, f));
         return GG_ERR_WORKSPACE;
     }
     cudaStream_t st = as_stream(stream);
@@ -469,12 +544,14 @@ int gg_postops_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t
     a.n = n; a.f = (int)f; a.mean = mean; a.invstd = invstd; a.gamma = gamma; a.act = act; a.slope = slope;
     a.l2 = l2norm; a.rownorm = const_cast<float*>(rownorm); a.train = train; a.dgamma = dgamma; a.dbeta = dbeta;
     a.partial = static_cast<float*>(workspace);
-    const bool vec = f % 4 == 0 && po_vec_ok(go, ld_go) && po_vec_ok(out, ld_out) && po_vec_ok(y, ld_y) && po_vec_ok(dy, ld_dy);
+    a.res_mode = mode; a.p = (int)p; a.dres = dres; a.ld_dres = ld_dres;
+    const bool vec = f % 4 == 0 && p % 4 == 0 && po_vec_ok(go, ld_go) && po_vec_ok(out, ld_out) && po_vec_ok(y, ld_y) &&
+                     po_vec_ok(dy, ld_dy) && po_vec_ok(dres, ld_dres);
     if (mean) {   // dgamma / dbeta (also in eval mode: the affine parameters still get gradients)
         int64_t chunk;
         const int blocks = po_chunks(n, &chunk);
         const size_t smem = (size_t)(kPoWarps * 2 + 2) * f * sizeof(float);
-        GG_REQUIRE(smem <= 200 * 1024, "gg_postops_bwd_f32: f=%lld too wide for the column reduction", (long long)f);
+        GG_REQUIRE(smem <= 200 * 1024, "%s: f=%lld too wide for the column reduction", who, (long long)f);
         if (vec) {
             GG_CUDA(cudaFuncSetAttribute(postops_bwd_reduce_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             postops_bwd_reduce_kernel<4><<<blocks, kPoThreads, smem, st>>>(a, chunk);
@@ -487,7 +564,7 @@ int gg_postops_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t
         GG_LAUNCHED();
     }
     const size_t smem_apply = (size_t)5 * f * sizeof(float);
-    GG_REQUIRE(smem_apply <= 200 * 1024, "gg_postops_bwd_f32: f=%lld too wide", (long long)f);
+    GG_REQUIRE(smem_apply <= 200 * 1024, "%s: f=%lld too wide", who, (long long)f);
     if (vec) {
         GG_CUDA(cudaFuncSetAttribute(postops_bwd_apply_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_apply));
         postops_bwd_apply_kernel<4><<<po_row_grid(n), kPoThreads, smem_apply, st>>>(a);
@@ -497,6 +574,48 @@ int gg_postops_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t
     }
     GG_LAUNCHED();
     return GG_OK;
+}
+
+int gg_postops_fwd_f32(const float* y, int64_t ld_y, int64_t n, int64_t f, const float* mean, const float* invstd,
+                       const float* gamma, const float* beta, int act, float slope, int l2norm, float* out,
+                       int64_t ld_out, float* rownorm, gg_stream_t stream) {
+    return po_fwd("gg_postops_fwd_f32", y, ld_y, nullptr, 0, n, f, 0, GG_SKIP_NONE, mean, invstd, gamma, beta, act, slope,
+                  l2norm, out, ld_out, rownorm, stream);
+}
+
+int gg_postops_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t ld_out, const float* y, int64_t ld_y,
+                       int64_t n, int64_t f, const float* mean, const float* invstd, const float* gamma, int train,
+                       int act, float slope, int l2norm, const float* rownorm, float* dy, int64_t ld_dy, float* dgamma,
+                       float* dbeta, void* workspace, size_t workspace_bytes, gg_stream_t stream) {
+    return po_bwd("gg_postops_bwd_f32", go, ld_go, out, ld_out, y, ld_y, n, f, 0, GG_SKIP_NONE, mean, invstd, gamma, train,
+                  act, slope, l2norm, rownorm, dy, ld_dy, nullptr, 0, dgamma, dbeta, workspace, workspace_bytes, stream);
+}
+
+static int po_skip_check(const char* who, int mode, int64_t p) {
+    GG_REQUIRE((mode == GG_SKIP_SUM && p == 0) || (mode == GG_SKIP_PREFIX && p >= 1 && p < ((int64_t)1 << 20)),
+               "%s: mode=%d with p=%lld (SUM takes p = 0, PREFIX 1 <= p < 2^20)", who, mode, (long long)p);
+    return GG_OK;
+}
+
+int gg_postops_skip_fwd_f32(const float* y, int64_t ld_y, const float* res, int64_t ld_res, int64_t n, int64_t f,
+                            int64_t p, int mode, const float* mean, const float* invstd, const float* gamma,
+                            const float* beta, int act, float slope, int l2norm, float* out, int64_t ld_out,
+                            float* rownorm, gg_stream_t stream) {
+    int rc = po_skip_check("gg_postops_skip_fwd_f32", mode, p);
+    if (rc != GG_OK) return rc;
+    return po_fwd("gg_postops_skip_fwd_f32", y, ld_y, res, ld_res, n, f, p, mode, mean, invstd, gamma, beta, act, slope,
+                  l2norm, out, ld_out, rownorm, stream);
+}
+
+int gg_postops_skip_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t ld_out, const float* y,
+                            int64_t ld_y, int64_t n, int64_t f, int64_t p, int mode, const float* mean,
+                            const float* invstd, const float* gamma, int train, int act, float slope, int l2norm,
+                            const float* rownorm, float* dy, int64_t ld_dy, float* dres, int64_t ld_dres, float* dgamma,
+                            float* dbeta, void* workspace, size_t workspace_bytes, gg_stream_t stream) {
+    int rc = po_skip_check("gg_postops_skip_bwd_f32", mode, p);
+    if (rc != GG_OK) return rc;
+    return po_bwd("gg_postops_skip_bwd_f32", go, ld_go, out, ld_out, y, ld_y, n, f, p, mode, mean, invstd, gamma, train,
+                  act, slope, l2norm, rownorm, dy, ld_dy, dres, ld_dres, dgamma, dbeta, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

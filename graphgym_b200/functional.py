@@ -377,6 +377,27 @@ def dot_attention_aggregate(h, bias, layout, agg):
     return _DotAttentionAgg.apply(h, bias, layout, agg)
 
 
+def _bn_forward(ctx, y, bn, training):
+    """-> (mean, invstd) the post-op kernels normalise with (None, None without BN), updating ``bn``'s running statistics
+    and num_batches_tracked as nn.BatchNorm1d would; sets ctx.train (batch statistics)."""
+    mean = invstd = None
+    if bn is not None:
+        if training or bn.running_mean is None:
+            mom = 0.0
+            if training and bn.running_mean is not None:
+                bn.num_batches_tracked += 1
+                mom = bn.momentum if bn.momentum is not None else 1.0 / float(bn.num_batches_tracked)
+            track = training and bn.running_mean is not None
+            mean, invstd = ops.bn_stats(y, bn.eps, bn.running_mean if track else None,
+                                        bn.running_var if track else None, mom)
+            ctx.train = True
+        else:
+            mean = bn.running_mean
+            invstd = torch.rsqrt(bn.running_var + bn.eps)   # [F]-sized, eval mode only
+            ctx.train = False
+    return mean, invstd
+
+
 class _PostOps(torch.autograd.Function):
     """out = l2norm( act( BatchNorm1d(y) ) ) in two kernels forward (statistics, apply) and two backward
     (column sums, apply) — ref: graphgym/models/layer.py:26-46, gnn.py:79-80."""
@@ -384,21 +405,7 @@ class _PostOps(torch.autograd.Function):
     @staticmethod
     def forward(ctx, y, gamma, beta, bn, training, act, slope, l2norm):
         y = y.contiguous()
-        mean = invstd = None
-        if bn is not None:
-            if training or bn.running_mean is None:
-                mom = 0.0
-                if training and bn.running_mean is not None:
-                    bn.num_batches_tracked += 1
-                    mom = bn.momentum if bn.momentum is not None else 1.0 / float(bn.num_batches_tracked)
-                track = training and bn.running_mean is not None
-                mean, invstd = ops.bn_stats(y, bn.eps, bn.running_mean if track else None,
-                                            bn.running_var if track else None, mom)
-                ctx.train = True
-            else:
-                mean = bn.running_mean
-                invstd = torch.rsqrt(bn.running_var + bn.eps)   # [F]-sized, eval mode only
-                ctx.train = False
+        mean, invstd = _bn_forward(ctx, y, bn, training)
         out, rownorm = ops.postops_fwd(y, mean, invstd, gamma, beta, act, slope, l2norm)
         ctx.act, ctx.slope, ctx.l2norm, ctx.has_bn = act, slope, l2norm, bn is not None
         ctx.save_for_backward(y, out, mean, invstd, gamma, rownorm)
@@ -419,3 +426,36 @@ def post_ops(y, bn=None, training=True, act=ops.ACT_NONE, slope=0.0, l2norm=Fals
     gamma = bn.weight if bn is not None else None
     beta = bn.bias if bn is not None else None
     return _PostOps.apply(y, gamma, beta, bn, bool(training), int(act), float(slope), bool(l2norm))
+
+
+class _SkipPostOps(torch.autograd.Function):
+    """The epilogue of a GraphGym skip block (ref: graphgym/models/gnn.py GNNSkipBlock, GNNSkipStage):
+    SKIP_SUM out = l2norm( act( BatchNorm1d(y) + res ) ), SKIP_PREFIX out = l2norm( act( cat([res, BatchNorm1d(y)], 1) ) )
+    in the post-op kernels, two forward (statistics, apply) and two backward (column sums, apply: dy and dres)."""
+
+    @staticmethod
+    def forward(ctx, y, res, gamma, beta, bn, training, act, slope, l2norm, mode):
+        y = y.contiguous()
+        mean, invstd = _bn_forward(ctx, y, bn, training)
+        out, rownorm = ops.postops_skip_fwd(y, res, mode, mean, invstd, gamma, beta, act, slope, l2norm)
+        ctx.act, ctx.slope, ctx.l2norm, ctx.mode = act, slope, l2norm, mode
+        ctx.save_for_backward(y, out, mean, invstd, gamma, rownorm)
+        return out
+
+    @staticmethod
+    def backward(ctx, go):
+        y, out, mean, invstd, gamma, rownorm = ctx.saved_tensors
+        dy, dres, dgamma, dbeta = ops.postops_skip_bwd(go.contiguous(), out, y, ctx.mode, mean, invstd, gamma,
+                                                       getattr(ctx, 'train', False), ctx.act, ctx.slope, ctx.l2norm,
+                                                       rownorm)
+        if gamma is None:
+            dgamma = dbeta = None
+        return dy, dres, dgamma, dbeta, None, None, None, None, None, None
+
+
+def skip_post_ops(y, res, mode, bn=None, training=True, act=ops.ACT_NONE, slope=0.0, l2norm=False):
+    """``mode``: ops.SKIP_SUM (skipsum: + res) or ops.SKIP_PREFIX (skipconcat: res as the leading columns).
+    ``bn``: an ``nn.BatchNorm1d`` on y (its parameters / buffers are used and updated as the module would) or None."""
+    gamma = bn.weight if bn is not None else None
+    beta = bn.bias if bn is not None else None
+    return _SkipPostOps.apply(y, res, gamma, beta, bn, bool(training), int(act), float(slope), bool(l2norm), int(mode))

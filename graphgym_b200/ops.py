@@ -760,6 +760,61 @@ def postops_bwd(go, out, y, mean, invstd, gamma, train, act, slope, l2norm, rown
     return dy, dgamma, dbeta
 
 
+SKIP_SUM, SKIP_PREFIX = 1, 2   # gg_skip: out = act(BN(y) + res) | out = act([res | BN(y)])
+
+
+def postops_skip_fwd(y, res, mode, mean, invstd, gamma, beta, act, slope, l2norm):
+    """The skip epilogue -> (out, rownorm or None).  SKIP_SUM: res [n, f], out [n, f]; SKIP_PREFIX: res [n, p],
+    out [n, p + f] with act(res) in the first p columns; the L2 (``l2norm``) over the whole output row."""
+    _need_cuda(y, res, mean, invstd, gamma, beta)
+    y, ld = _rows(y, "y")
+    res, ld_res = _rows(res, "res")
+    n, f = y.shape
+    if res.size(0) != n:
+        raise ValueError(f"postops_skip_fwd: res has {res.size(0)} rows, y {n}")
+    if mode == SKIP_SUM:
+        if res.size(1) != f:
+            raise ValueError(f"postops_skip_fwd: a sum skip needs res [n, {f}], got {tuple(res.shape)}")
+        p = 0
+    elif mode == SKIP_PREFIX:
+        p = res.size(1)
+    else:
+        raise ValueError(f"postops_skip_fwd: mode={mode}")
+    out = torch.empty((n, p + f), dtype=torch.float32, device=y.device)
+    rownorm = torch.empty(max(n, 1), dtype=torch.float32, device=y.device)[:n] if l2norm else None
+    check(lib().gg_postops_skip_fwd_f32(_ptr(y), ld, _ptr(res), ld_res, n, f, p, int(mode), _ptr(mean), _ptr(invstd),
+                                        _ptr(gamma), _ptr(beta), int(act), float(slope), int(bool(l2norm)), _ptr(out),
+                                        max(p + f, 1), _ptr(rownorm), _stream()), "gg_postops_skip_fwd_f32")
+    return out, rownorm
+
+
+def postops_skip_bwd(go, out, y, mode, mean, invstd, gamma, train, act, slope, l2norm, rownorm):
+    """-> (dy, dres, dgamma or None, dbeta or None) of ``postops_skip_fwd``; the prefix width is out's width - y's."""
+    _need_cuda(go, out, y)
+    go, ld_go = _rows(go, "go")
+    out, ld_o = _rows(out, "out")
+    y, ld_y = _rows(y, "y")
+    n, f = y.shape
+    p = out.size(1) - f if mode == SKIP_PREFIX else 0
+    dev = go.device
+    dy = torch.empty((n, f), dtype=torch.float32, device=dev)
+    dres = torch.empty((n, p if mode == SKIP_PREFIX else f), dtype=torch.float32, device=dev)
+    dgamma = dbeta = ws = None
+    ws_bytes = 0
+    L = lib()
+    if mean is not None:
+        dgamma = torch.empty(f, dtype=torch.float32, device=dev)
+        dbeta = torch.empty(f, dtype=torch.float32, device=dev)
+        ws_bytes = int(L.gg_postops_workspace_bytes(n, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    check(L.gg_postops_skip_bwd_f32(_ptr(go), ld_go, _ptr(out), ld_o, _ptr(y), ld_y, n, f, p, int(mode), _ptr(mean),
+                                    _ptr(invstd), _ptr(gamma), int(bool(train)), int(act), float(slope),
+                                    int(bool(l2norm)), _ptr(rownorm), _ptr(dy), max(f, 1), _ptr(dres),
+                                    max(dres.size(1), 1), _ptr(dgamma), _ptr(dbeta), _ptr(ws), ws_bytes, _stream()),
+          "gg_postops_skip_bwd_f32")
+    return dy, dres, dgamma, dbeta
+
+
 # --------------------------------------------------------------------------------------------
 # GAT
 # --------------------------------------------------------------------------------------------

@@ -552,6 +552,24 @@ int gg_postops_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t
                        int act, float slope, int l2norm, const float* rownorm, float* dy, int64_t ld_dy, float* dgamma,
                        float* dbeta, void* workspace, size_t workspace_bytes, gg_stream_t stream);
 
+/* The skip epilogue of GNNSkipBlock (ref: graphgym/models/gnn.py GNNSkipBlock / GNNSkipStage) on the same kernels: the
+ * last layer's BatchNorm, the skip connection, the stage activation and (last block) the stage's L2 in one pass.
+ *   GG_SKIP_SUM     (skipsum, p = 0)     out [n, f]      = l2?(act(BN(y) + res)),  res [n, f]
+ *   GG_SKIP_PREFIX  (skipconcat, p >= 1) out [n, p + f]  = l2?([act(res) | act(BN(y))]),  res [n, p]; the L2 over p + f
+ * gg_postops_skip_bwd_f32: as gg_postops_bwd_f32 (gates from the SAVED out, go / out rows p + f wide in PREFIX mode), and
+ *   dres = dA, the gradient at the activation's input: the f columns (SUM) or the p carried columns (PREFIX);
+ *   dgamma / dbeta sum over the f columns only.  Statistics: gg_bn_stats_f32 of y; workspace as gg_postops_bwd_f32. */
+enum gg_skip { GG_SKIP_NONE = 0, GG_SKIP_SUM = 1, GG_SKIP_PREFIX = 2 };
+int gg_postops_skip_fwd_f32(const float* y, int64_t ld_y, const float* res, int64_t ld_res, int64_t n, int64_t f,
+                            int64_t p, int mode, const float* mean, const float* invstd, const float* gamma,
+                            const float* beta, int act, float slope, int l2norm, float* out, int64_t ld_out,
+                            float* rownorm, gg_stream_t stream);
+int gg_postops_skip_bwd_f32(const float* go, int64_t ld_go, const float* out, int64_t ld_out, const float* y,
+                            int64_t ld_y, int64_t n, int64_t f, int64_t p, int mode, const float* mean,
+                            const float* invstd, const float* gamma, int train, int act, float slope, int l2norm,
+                            const float* rownorm, float* dy, int64_t ld_dy, float* dres, int64_t ld_dres, float* dgamma,
+                            float* dbeta, void* workspace, size_t workspace_bytes, gg_stream_t stream);
+
 /* Per-row softmax over GIVEN per-slot logits and its backward — the scaled dot-product scorer of the Tfg GAT variant
  * (ref: TfgIDLayer.py:336-345, sparse_adj.py:136-151): alpha[s] = exp(scale z[s] - max_row) / sum_row;
  * dz[s] = scale alpha[s] (dalpha[s] - sum_row alpha dalpha).  The logits come from gg_gat_sddmm_mp_f32 (<Q_i, K_j>). */
