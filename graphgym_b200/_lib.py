@@ -82,6 +82,20 @@ SIGNATURES = {
                                     c_i64, c_f32, c_ptr, c_ptr]),
     "gg_spmm_row_max_bwd_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_f32,
                                         c_ptr, c_i64, c_ptr]),
+    "gg_edge_row_reduce_f32": (c_int, [c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_int, c_ptr, c_i64, c_ptr]),
+    "gg_edge_rows_self_f32": (c_int, [c_ptr, c_i64, c_i64, c_int, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64,
+                                      c_ptr]),
+    "gg_max_mask_f32": (c_int, [c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_ptr, c_i64, c_ptr]),
+    "gg_edge_max_sell_f32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64,
+                                     c_ptr, c_i64, c_ptr, c_i64, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64,
+                                     c_i64, c_ptr, c_i64, c_f32, c_ptr, c_ptr, c_size, c_int, c_ptr]),
+    "gg_edge_max_row_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_ptr, c_i64,
+                                    c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_ptr, c_i64, c_f32, c_ptr, c_ptr]),
+    "gg_edge_max_winner_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_i64, c_ptr,
+                                       c_i64, c_ptr]),
+    "gg_edge_max_wgrad_workspace_bytes": (c_size, [c_i64, c_i64, c_i64]),
+    "gg_edge_max_wgrad_f32": (c_int, [c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_i64, c_ptr, c_i64,
+                                      c_ptr, c_size, c_ptr]),
     "gg_max_winner_sddmm_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_int, c_i64, c_ptr,
                                         c_ptr]),
     "gg_gat_alpha_heads_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_f32, c_ptr, c_ptr]),

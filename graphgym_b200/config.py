@@ -23,10 +23,10 @@ def _defaults():
     c.gnn = _Node(layers_pre_mp=0, layers_mp=2, layers_post_mp=0, dim_inner=16, layer_type='generalconv',
                   stage_type='stack', batchnorm=True, act='relu', dropout=0.0, agg='add',
                   normalize_adj=False, l2norm=True, keep_edge=0.5, self_msg='concat', att_heads=1,
-                  skip_every=1)
+                  skip_every=1, msg_direction='single')
     c.bn = _Node(eps=1e-5, mom=0.1)
     c.mem = _Node(inplace=False)
-    c.dataset = _Node(transform='none', augment_feature=[], augment_feature_dims=[])
+    c.dataset = _Node(transform='none', augment_feature=[], augment_feature_dims=[], edge_dim=128)
     c.train = _Node(batch_size=16)
     c.num_threads = 6
     c.device = 'auto'

@@ -89,6 +89,99 @@ def aggregate(x, layout, kind="sum", self_scale=0.0, bias=None, residual=None):
     return _Aggregate.apply(x, layout, kind, float(self_scale), bias, half, residual)
 
 
+class _EdgeAggregate(torch.autograd.Function):
+    """out[i] = A h_j + r_i h_i + (S a)[i] W_a^T (+ residual[i] + bias): the add / mean aggregation of the messages
+    h_j[j] (+ h_i[i]) + a_e W_a^T, which is linear, so no per-edge message is formed.  A = the sum or mean over the
+    in-edges, S a = the per-target sum or mean of the edge-feature rows, r_i = indeg(i) (add) or [indeg(i) > 0] (mean)."""
+
+    @staticmethod
+    def forward(ctx, h_j, h_i, a, w_a, layout, kind, bias, residual):
+        csr = layout.csr
+        mean = kind == "mean"
+        sa = ops.edge_row_reduce(csr, a, mean)
+        t = ops.id_gemm([(sa, w_a, None)], csr.num_nodes, w_a.size(0), b_trans=True)       # (S a) W_a^T
+        w_fwd, _ = layout.weights(kind)
+        out = ops.spmm(csr, h_j.contiguous(), w_fwd, ops.MEAN if mean else ops.SUM, t, 1.0, bias)
+        if h_i is not None or residual is not None:
+            ops.edge_rows_self(csr, h_i, y=out, z=residual, mean=mean)
+        ctx.layout, ctx.kind = layout, kind
+        ctx.has_hi, ctx.has_bias, ctx.has_residual = h_i is not None, bias is not None, residual is not None
+        ctx.save_for_backward(sa, w_a)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        sa, w_a = ctx.saved_tensors
+        g = g.contiguous()
+        lay = ctx.layout
+        csr = lay.csr
+        mean = ctx.kind == "mean"
+        ghj = ghi = ga = gw = gb = None
+        if ctx.needs_input_grad[0]:
+            _, w_bwd = lay.weights(ctx.kind)
+            ghj = ops.spmm(lay.csc, g, w_bwd, ops.SUM, None, 0.0, None)
+        if ctx.has_hi and ctx.needs_input_grad[1]:
+            ghi = ops.edge_rows_self(csr, g, mean=mean)
+        if ctx.needs_input_grad[2]:
+            # d a_e = (g W_a)[target(e)] (/ indeg for the mean), in edge order
+            gwa = ops.id_gemm([(g, w_a, None)], csr.num_nodes, w_a.size(1))
+            if mean:
+                ops.rows_epilogue(gwa, csr, out=gwa)
+            ga = ops.gather_rows(gwa, lay.edge_index[1])
+        if ctx.needs_input_grad[3]:
+            gw = ops.gemm_tn(g, sa)
+        if ctx.has_bias and ctx.needs_input_grad[6]:
+            gb = ops.colsum(g)
+        return ghj, ghi, ga, gw, None, None, gb, (g if ctx.has_residual else None)
+
+
+class _EdgeAggregateMax(torch.autograd.Function):
+    """out[i,c] = max_{e = (j -> i)} h_j[j,c] (+ h_i[i,c]) + a_e . W_a[c] (0 without in-edges) + residual[i,c] + bias[c];
+    the gradient goes to the first in-edge (in edge order) that reaches the maximum, per column.  The edge term is formed
+    per edge inside the reduction (``ops.edge_max``) and never stored."""
+
+    @staticmethod
+    def forward(ctx, h_j, h_i, a, w_a, layout, bias, residual):
+        out, arg = ops.edge_max(layout.csr, h_j, h_i, a, w_a, residual, 1.0 if residual is not None else 0.0, bias)
+        ctx.layout = layout
+        ctx.has_hi, ctx.has_bias, ctx.has_residual = h_i is not None, bias is not None, residual is not None
+        ctx.save_for_backward(a, w_a, arg)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        a, w_a, arg = ctx.saved_tensors
+        g = g.contiguous()
+        lay = ctx.layout
+        ghj = ghi = ga = gw = gb = None
+        if ctx.needs_input_grad[0]:
+            ghj = ops.spmm_max_bwd(lay.csc, lay.csc2csr, g, arg)
+        if ctx.has_hi and ctx.needs_input_grad[1]:
+            ghi = ops.max_mask(g, arg)
+        if ctx.needs_input_grad[2]:
+            ga = ops.edge_max_winner(lay.csr, arg, g, w_a)
+        if ctx.needs_input_grad[3]:
+            gw = ops.edge_max_wgrad(lay.csr, arg, g, a)
+        if ctx.has_bias and ctx.needs_input_grad[5]:
+            gb = ops.colsum(g)
+        return ghj, ghi, ga, gw, None, gb, (g if ctx.has_residual else None)
+
+
+def edge_aggregate(h_j, h_i, edge_feature, w_a, layout, agg, bias=None, residual=None):
+    """Aggregation of the edge-feature messages m_e = h_j[j] (+ h_i[i]) + edge_feature[e] w_a^T over the in-edges
+    e = (j -> i) of ``layout`` (edge order = the layout's edge_index), + residual + bias.  ``agg``: 'add' | 'mean' | 'max'
+    (max: 0 for a row without in-edges, the gradient to the first in-edge reaching each column's maximum).  ``h_i`` may
+    be None; ``w_a``: [f, edge_dim] (a column slice of nn.Linear's weight).  fp32 only."""
+    from .config import cfg
+    if cfg.b200.gather_dtype == "bf16":
+        raise NotImplementedError("cfg.b200.gather_dtype = 'bf16' has no edge-feature aggregation")
+    if agg == "max":
+        return _EdgeAggregateMax.apply(h_j, h_i, edge_feature, w_a, layout, bias, residual)
+    if agg not in ("add", "mean"):
+        raise NotImplementedError("edge_aggregate: agg {!r}".format(agg))
+    return _EdgeAggregate.apply(h_j, h_i, edge_feature, w_a, layout, "mean" if agg == "mean" else "sum", bias, residual)
+
+
 class _SegLinear(torch.autograd.Function):
     """out = act( sum_g diag(c_g) X_g W_g + bias ).
 

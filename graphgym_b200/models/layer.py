@@ -194,6 +194,8 @@ _builtin = {
     'gatconv': GATConv,
     'ginconv': GINConv,
     'generalconv': _generalconv.GeneralConv,
+    'generaledgeconv': _generalconv.GeneralEdgeConv,
+    'generalsampleedgeconv': _generalconv.GeneralSampleEdgeConv,
 }
 
 # built-ins win on a name clash, contrib registrations fill the rest (ref: layer.py:238)
@@ -213,9 +215,11 @@ def resolve_layer(name):
 
 
 class Batch:
-    """Minimal stand-in for a DeepSNAP batch: the three attributes the layers touch."""
+    """Minimal stand-in for a DeepSNAP batch: the attributes the layers touch (``edge_feature``: [E, edge_dim] rows in
+    edge_index order, read by the edge-feature layers)."""
 
-    def __init__(self, node_feature, edge_index, node_id_index=None):
+    def __init__(self, node_feature, edge_index, node_id_index=None, edge_feature=None):
         self.node_feature = node_feature
         self.edge_index = edge_index
         self.node_id_index = node_id_index
+        self.edge_feature = edge_feature

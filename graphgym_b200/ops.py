@@ -464,6 +464,140 @@ def max_winner_sddmm(csr, arg, g, h, heads=1):
     return dalpha
 
 
+EDGE_MAX_KD = 256   # edge_dim limit of edge_max (its W_a column tile is staged in shared memory)
+
+
+def _edge_rows(a, name):
+    if a.dtype != torch.float32 or a.dim() != 2:
+        raise ValueError(f"{name}: expected a 2-D float32 tensor, got {tuple(a.shape)} {a.dtype}")
+    return _rows(a, name)
+
+
+def edge_row_reduce(csr, a, mean=False):
+    """[n, kd]: out[i] = sum over the CSR slots s of row i of a[perm[s]] (slot order), / indeg(i) with ``mean``; rows
+    without slots 0.  ``a``: [E, kd] in edge order (csrc/edge_agg.cu)."""
+    _need_cuda(a, csr.rowptr)
+    a, lda = _edge_rows(a, "edge_feature")
+    n, k = csr.num_nodes, a.size(1)
+    out = _f32((n, k), a.device)
+    check(lib().gg_edge_row_reduce_f32(_ptr(csr.rowptr), _ptr(csr.perm), n, _ptr(a), lda, k, int(bool(mean)), _ptr(out),
+                                       max(k, 1), _stream()), "gg_edge_row_reduce_f32")
+    return out
+
+
+def edge_rows_self(csr, h=None, y=None, z=None, mean=False):
+    """y + r * h + z per row (each term optional), r = indeg(i) or, with ``mean``, [indeg(i) > 0]; written into ``y``
+    when given."""
+    _need_cuda(h, y, z, csr.rowptr)
+    n = csr.num_nodes
+    ldh = ldy = ldz = 0
+    if h is not None:
+        h, ldh = _rows(h, "h")
+    if z is not None:
+        z, ldz = _rows(z, "z")
+    f = next(t.size(1) for t in (h, y, z) if t is not None)
+    if y is not None:
+        y_t, ldy = _rows(y, "y")
+        assert y_t is y
+        out, ldo = y, ldy
+    else:
+        out, ldo = _f32((n, f), csr.rowptr.device), max(f, 1)
+    check(lib().gg_edge_rows_self_f32(_ptr(csr.rowptr), n, f, int(bool(mean)), _ptr(y), ldy, _ptr(h), ldh, _ptr(z), ldz,
+                                      _ptr(out), ldo, _stream()), "gg_edge_rows_self_f32")
+    return out
+
+
+def max_mask(g, arg):
+    """g where arg >= 0, else 0."""
+    _need_cuda(g, arg)
+    g, ldg = _rows(g, "g")
+    arg = arg.contiguous()
+    n, f = g.shape
+    out = _f32((n, f), g.device)
+    check(lib().gg_max_mask_f32(_ptr(g), ldg, _ptr(arg), f, n, f, _ptr(out), max(f, 1), _stream()), "gg_max_mask_f32")
+    return out
+
+
+def edge_max(csr, h_j, h_i, a, w_a, x_self=None, self_scale=0.0, bias=None, algo=None):
+    """Max aggregation with the edge term -> (out [n, f], arg int32 [n, f]):
+    out[i,c] = max_{s in row i} h_j[nbr[s],c] + a[perm[s]] . w_a[c] (+ h_i[i,c] where the row has a slot; 0 for an empty
+    row) + self_scale*x_self + bias; arg = the first slot reaching the maximum, -1 for an empty row.  ``h_i`` may be None;
+    ``w_a``: [f, kd] (rows may be strided, e.g. a column slice of nn.Linear's weight).  Path choice as ``spmm_max``;
+    ``algo`` ('sell' | 'row') overrides it."""
+    _need_cuda(h_j, h_i, a, w_a, x_self, bias, csr.rowptr)
+    h_j, ldj = _rows(h_j, "h_j")
+    a, lda = _edge_rows(a, "edge_feature")
+    w_a, ldw = _rows(w_a, "w_a")
+    n, f, kd = csr.num_nodes, h_j.size(1), a.size(1)
+    if kd > EDGE_MAX_KD:
+        raise NotImplementedError(f"edge_max: edge_dim {kd} > {EDGE_MAX_KD}")
+    dev = h_j.device
+    out = _f32((n, f), dev)
+    arg = torch.empty((n, f), dtype=torch.int32, device=dev)
+    if n == 0 or f == 0:
+        return out, arg
+    ldi = ld_self = 0
+    if h_i is not None:
+        h_i, ldi = _rows(h_i, "h_i")
+    if x_self is not None:
+        x_self, ld_self = _rows(x_self, "x_self")
+    if bias is not None:
+        bias = bias.contiguous()
+    L = lib()
+    aligned = (f % 4 == 0 and ldj % 4 == 0 and _al16(h_j) and _al16(bias) and
+               (h_i is None or (ldi % 4 == 0 and _al16(h_i))) and (x_self is None or (ld_self % 4 == 0 and _al16(x_self))))
+    if algo is None:
+        algo = "sell" if aligned and n + csr.num_slots >= 1 << 14 else "row"
+    if algo == "sell":
+        if not aligned:
+            raise ValueError("edge_max: the sliced-ELL kernel needs f % 4 == 0 and 16-byte aligned rows")
+        sl = sell_layout(csr)
+        ws_bytes = int(L.gg_spmm_sell_max_workspace_bytes(sl.partial_rows, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        check(L.gg_edge_max_sell_f32(_ptr(sl.chunk_ptr), sl.chunks, _ptr(sl.idx), _ptr(sl.slot_of), _ptr(csr.perm),
+                                     _ptr(sl.vdst), _ptr(sl.hub_rows), _ptr(sl.hub_pptr), sl.hubs, sl.partial_rows,
+                                     _ptr(h_j), ldj, _ptr(h_i), ldi, _ptr(a), lda, kd, _ptr(w_a), ldw, _ptr(out), f,
+                                     _ptr(arg), f, n, f, _ptr(x_self), ld_self, float(self_scale), _ptr(bias), _ptr(ws),
+                                     ws_bytes, _spmm_flags(), _stream()), "gg_edge_max_sell_f32")
+    elif algo == "row":
+        check(L.gg_edge_max_row_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(csr.perm), _ptr(h_j), ldj, _ptr(h_i), ldi, _ptr(a),
+                                    lda, kd, _ptr(w_a), ldw, _ptr(out), f, _ptr(arg), f, n, f, _ptr(x_self), ld_self,
+                                    float(self_scale), _ptr(bias), _stream()), "gg_edge_max_row_f32")
+    else:
+        raise ValueError(f"edge_max: algo={algo!r}")
+    return out, arg
+
+
+def edge_max_winner(csr, arg, g, w_a):
+    """d edge_feature [E, kd] of ``edge_max``: row perm[s] = sum over the columns c slot s won of g[i,c] w_a[c], in
+    column order; 0 for an edge that won nothing."""
+    _need_cuda(arg, g, w_a, csr.rowptr)
+    g, ldg = _rows(g, "g")
+    w_a, ldw = _rows(w_a, "w_a")
+    arg = arg.contiguous()
+    n, f, kd = csr.num_nodes, g.size(1), w_a.size(1)
+    da = _f32((csr.num_edges, kd), g.device)
+    check(lib().gg_edge_max_winner_f32(_ptr(csr.rowptr), _ptr(csr.perm), _ptr(arg), f, _ptr(g), ldg, _ptr(w_a), ldw, n, f,
+                                       kd, _ptr(da), max(kd, 1), _stream()), "gg_edge_max_winner_f32")
+    return da
+
+
+def edge_max_wgrad(csr, arg, g, a):
+    """d w_a [f, kd] of ``edge_max``: sum_i g[i,c] a[perm[arg[i,c]]] over the rows with arg >= 0 (fixed order)."""
+    _need_cuda(arg, g, a, csr.rowptr)
+    g, ldg = _rows(g, "g")
+    a, lda = _edge_rows(a, "edge_feature")
+    arg = arg.contiguous()
+    n, f, kd = csr.num_nodes, g.size(1), a.size(1)
+    L = lib()
+    dw = _f32((f, kd), g.device)
+    ws_bytes = int(L.gg_edge_max_wgrad_workspace_bytes(n, f, kd))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=g.device)
+    check(L.gg_edge_max_wgrad_f32(_ptr(csr.perm), _ptr(arg), f, _ptr(g), ldg, _ptr(a), lda, n, f, kd, _ptr(dw), max(kd, 1),
+                                  _ptr(ws), ws_bytes, _stream()), "gg_edge_max_wgrad_f32")
+    return dw
+
+
 def rows_epilogue(x, mean_csr=None, rank1=None, heads=1, bias=None, out=None):
     """out[i, :] = x[i, :] / indeg(i) (with ``mean_csr``; rows without in-edges unscaled) + s1[i, k] v1 + s2[i, k] v2
     (``rank1`` = (s1 [n, heads], v1 [f], s2, v2), k the column's head) + bias.  ``out`` may be ``x``."""

@@ -265,6 +265,53 @@ int gg_spmm_row_max_bwd_f32(const int32_t* rowptr, const int32_t* nbr, const int
                             const float* g, int64_t ldg, const int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
                             float self_scale, float* dx, int64_t ldd, gg_stream_t stream);
 
+/* Edge-feature message passing (csrc/edge_agg.cu; generaledgeconv / generalsampleedgeconv).  The message on edge
+ * e = (j -> i), CSR slot s, perm[s] = e, is h_j[j] (+ h_i[i]) + a[e] W_a^T, a the [E, kd] edge features, W_a [f, kd].
+ *   gg_edge_row_reduce_f32    out[i,k] = sum over the slots s of row i of a[perm[s],k], in slot order; / indeg(i) with
+ *                             `mean` (rows without slots 0)
+ *   gg_edge_rows_self_f32     out[i,c] = y[i,c] + r_i h[i,c] + z[i,c] (y, h, z nullable: 0), r_i = indeg(i) or, with
+ *                             `mean`, [indeg(i) > 0]; element-wise, out may alias y
+ *   gg_max_mask_f32           out[i,c] = arg[i,c] >= 0 ? g[i,c] : 0
+ *   gg_edge_max_sell_f32 / gg_edge_max_row_f32
+ *                             out[i,c] = max over the slots s of row i of h_j[nbr[s],c] + sum_k a[perm[s],k] W_a[c,k],
+ *                             + h_i[i,c] (nullable), 0 for a row without slots; + self_scale x_self[i,c] + bias[c];
+ *                             arg[i,c] = the first slot reaching the maximum (strict `>` in slot order, -1 for an empty
+ *                             row).  The sliced-ELL entry takes the CSR's gg_sell_build layout (flags bit 2 as in
+ *                             gg_spmm_sell_f32), f % 4 == 0, 16-byte aligned rows, workspace
+ *                             gg_spmm_sell_max_workspace_bytes(partial rows, f); the row entry takes the plain CSR and any
+ *                             f.  Both need kd <= 256 (GG_ERR_UNSUPPORTED) and give the same bits.
+ *   gg_edge_max_winner_f32    da[perm[s],k] = sum over the columns c with arg[i,c] == s (s a slot of row i) of
+ *                             g[i,c] W_a[c,k], in column order; 0 for an edge that won no column.  Every edge of the
+ *                             layout is written once.
+ *   gg_edge_max_wgrad_f32     dw[c,k] = sum_i g[i,c] a[perm[arg[i,c]],k] over the rows with arg >= 0; per-block partials
+ *                             summed in a fixed order.  Workspace: gg_edge_max_wgrad_workspace_bytes(num_rows, f, kd).
+ * All are bitwise run-to-run deterministic (no atomics on data). */
+int gg_edge_row_reduce_f32(const int32_t* rowptr, const int32_t* perm, int64_t num_rows, const float* a, int64_t lda,
+                           int64_t k, int mean, float* out, int64_t ldo, gg_stream_t stream);
+int gg_edge_rows_self_f32(const int32_t* rowptr, int64_t num_rows, int64_t f, int mean, const float* y, int64_t ldy,
+                          const float* h, int64_t ldh, const float* z, int64_t ldz, float* out, int64_t ldo,
+                          gg_stream_t stream);
+int gg_max_mask_f32(const float* g, int64_t ldg, const int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
+                    float* out, int64_t ldo, gg_stream_t stream);
+int gg_edge_max_sell_f32(const uint32_t* chunk_ptr, int64_t chunks, const int32_t* idx, const int32_t* slot_of,
+                         const int32_t* perm, const int32_t* vdst, const int32_t* hub_rows, const int32_t* hub_pptr,
+                         int64_t hubs, int64_t partial_rows, const float* h_j, int64_t ldj, const float* h_i, int64_t ldi,
+                         const float* a, int64_t lda, int64_t kd, const float* w_a, int64_t ldw, float* out, int64_t ldo,
+                         int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f, const float* x_self, int64_t ld_self,
+                         float self_scale, const float* bias, void* workspace, size_t workspace_bytes, int flags,
+                         gg_stream_t stream);
+int gg_edge_max_row_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* perm, const float* h_j, int64_t ldj,
+                        const float* h_i, int64_t ldi, const float* a, int64_t lda, int64_t kd, const float* w_a,
+                        int64_t ldw, float* out, int64_t ldo, int32_t* arg, int64_t ld_arg, int64_t num_rows, int64_t f,
+                        const float* x_self, int64_t ld_self, float self_scale, const float* bias, gg_stream_t stream);
+int gg_edge_max_winner_f32(const int32_t* rowptr, const int32_t* perm, const int32_t* arg, int64_t ld_arg, const float* g,
+                           int64_t ldg, const float* w_a, int64_t ldw, int64_t num_rows, int64_t f, int64_t kd, float* da,
+                           int64_t ldda, gg_stream_t stream);
+size_t gg_edge_max_wgrad_workspace_bytes(int64_t num_rows, int64_t f, int64_t kd);
+int gg_edge_max_wgrad_f32(const int32_t* perm, const int32_t* arg, int64_t ld_arg, const float* g, int64_t ldg,
+                          const float* a, int64_t lda, int64_t num_rows, int64_t f, int64_t kd, float* dw, int64_t lddw,
+                          void* workspace, size_t workspace_bytes, gg_stream_t stream);
+
 /* Mean / max aggregation of the attention layers (csrc/attn_agg.cu; gaddconv / gmulconv with cfg.gnn.agg = 'mean' /
  * 'max').  heads H splits f into H blocks of c = f / H columns; column col belongs to head col / c.
  *   gg_max_winner_sddmm_f32   dalpha[s*H + k] = sum over the columns col of head k with arg[i,col] == s (s a slot of CSR
