@@ -96,6 +96,18 @@ SIGNATURES = {
     "gg_edge_max_wgrad_workspace_bytes": (c_size, [c_i64, c_i64, c_i64]),
     "gg_edge_max_wgrad_f32": (c_int, [c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_i64, c_ptr, c_i64,
                                       c_ptr, c_size, c_ptr]),
+    "gg_spline_spread_sell_f32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                          c_i64, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_int, c_ptr, c_size, c_int,
+                                          c_ptr]),
+    "gg_spline_blend_sell_f32": (c_int, [c_ptr, c_i64, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr,
+                                         c_i64, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_int, c_ptr, c_i64, c_ptr,
+                                         c_ptr, c_size, c_int, c_ptr]),
+    "gg_spline_spread_row_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_int,
+                                         c_ptr]),
+    "gg_spline_blend_row_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_i64, c_int,
+                                        c_ptr, c_i64, c_ptr, c_ptr]),
+    "gg_spline_du_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_ptr, c_i64, c_i64, c_i64, c_i64, c_ptr,
+                                 c_ptr]),
     "gg_max_winner_sddmm_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_ptr, c_i64, c_ptr, c_i64, c_i64, c_int, c_i64, c_ptr,
                                         c_ptr]),
     "gg_gat_alpha_heads_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_f32, c_ptr, c_ptr]),

@@ -182,6 +182,80 @@ def edge_aggregate(h_j, h_i, edge_feature, w_a, layout, agg, bias=None, residual
     return _EdgeAggregate.apply(h_j, h_i, edge_feature, w_a, layout, "mean" if agg == "mean" else "sum", bias, residual)
 
 
+class _SplineAggregate(torch.autograd.Function):
+    """out[i] = mean over e = (j -> i) of (c0_e x_j W0 + c1_e x_j W1) + x_i root + bias, (c0_e, c1_e) the degree-1 open
+    B-spline coefficients of u_e (kernel size 2).  No per-edge message is formed; two factorisations:
+      aggregate first  [P0 | P1] = spread(x) on the CSR, out = [P0 | P1 | x] [W0; W1; root] + bias (one GEMM);
+                       dX = blend([dP0 | dP1] = g [W0 | W1]^T) on the CSC + g root^T, dW_k = P_k^T g
+      transform first  H = x [W0 | W1], out = blend(H) on the CSR + x root + bias;
+                       [dH0 | dH1] = spread(g) on the CSC, dX = [dH0 | dH1] [W0 | W1]^T + g root^T, dW_k = x^T dH_k
+    On the CSC the slots carry 1/indeg(target).  d u (only when asked for) comes from a warp-per-row pass over the CSR."""
+
+    @staticmethod
+    def forward(ctx, x, u, weight, root, bias, layout, aggregate_first):
+        csr = layout.csr
+        x = x.contiguous()
+        uf = u.reshape(-1)
+        n, (fin, fout) = x.size(0), root.shape
+        if aggregate_first:
+            t = ops.spline_spread(csr, x, uf, mean=True)                                    # [P0 | P1]
+            w01 = weight.reshape(2 * fin, fout)                                              # [W0; W1]
+            out = ops.id_gemm([(t, w01, None), (x, root, None)], n, fout, bias=bias)
+        else:
+            w01 = torch.cat([weight[0], weight[1]], dim=1)                                   # [W0 | W1]
+            t = ops.id_gemm([(x, w01, None)], n, 2 * fout)                                   # [H0 | H1]
+            r = ops.id_gemm([(x, root, None)], n, fout)
+            out = ops.spline_blend(csr, t, uf, mean=True, residual=r, bias=bias)
+        ctx.layout, ctx.aggregate_first, ctx.u_shape = layout, aggregate_first, u.shape
+        ctx.has_bias = bias is not None
+        ctx.save_for_backward(x, uf, w01, root, t)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        x, uf, w01, root, t = ctx.saved_tensors
+        g = g.contiguous()
+        lay = ctx.layout
+        n, (fin, fout) = x.size(0), root.shape
+        _, w_csc = lay.weights("mean")                                                       # 1/indeg(target) per CSC slot
+        gx = gu = gw = groot = gb = None
+        need_x, need_u, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1], ctx.needs_input_grad[2]
+        if ctx.aggregate_first:
+            if need_x or need_u:
+                dp = ops.id_gemm([(g, w01, None)], n, 2 * fin, b_trans=True)                 # [dP0 | dP1]
+                if need_x:
+                    gx = ops.spline_blend(lay.csc, dp, uf, w_csc,
+                                          residual=ops.id_gemm([(g, root, None)], n, fin, b_trans=True))
+                if need_u:
+                    gu = ops.spline_du(lay.csr, uf, dp, fin, x, 0, fin)
+            if need_w:
+                gw = ops.gemm_tn(t, g).view(2, fin, fout)
+        else:
+            if need_x or need_w:
+                dh = ops.spline_spread(lay.csc, g, uf, w_csc)                                # [dH0 | dH1]
+                if need_x:
+                    gx = ops.id_gemm([(dh, w01, None), (g, root, None)], n, fin, b_trans=True)
+                if need_w:
+                    dw = ops.gemm_tn(x, dh)
+                    gw = torch.stack([dw[:, :fout], dw[:, fout:]])
+            if need_u:
+                gu = ops.spline_du(lay.csr, uf, g, 0, t, fout, fout)
+        if ctx.needs_input_grad[3]:
+            groot = ops.gemm_tn(x, g)
+        if ctx.has_bias and ctx.needs_input_grad[4]:
+            gb = ops.colsum(g)
+        if gu is not None:
+            gu = gu.view(ctx.u_shape)
+        return gx, gu, gw, groot, gb, None, None
+
+
+def spline_aggregate(x, pseudo, weight, root, bias, layout, aggregate_first):
+    """SplineConv's mean aggregation with the root weight (dim 1, kernel size 2, degree 1, open spline): ``pseudo`` the
+    [E] or [E, 1] float32 pseudo-coordinates in the edge order of ``layout``, ``weight`` [2, in, out], ``root`` [in, out].
+    ``aggregate_first`` picks the factorisation (the narrower side is gathered: in <= out aggregates first)."""
+    return _SplineAggregate.apply(x, pseudo, weight, root, bias, layout, bool(aggregate_first))
+
+
 class _SegLinear(torch.autograd.Function):
     """out = act( sum_g diag(c_g) X_g W_g + bias ).
 

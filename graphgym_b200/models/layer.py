@@ -10,7 +10,11 @@ neither vendored nor a dependency here, so each layer restates the PyG module's 
     GINConv   nn((1 + eps) x_i + sum_j x_j), eps = 0 buffer, loops kept
     GATConv   remove + add self loops, additive attention (slope 0.2, heads=1), edge-softmax fused
               into the aggregation (parameters weight / att / bias as in PyG <= 1.5 and idconv.py)
+    SplineConv  PyG 1.6 SplineConv(dim=1, kernel_size=2): the mean over the in-edges of the degree-1 open B-spline
+              weighting of the pseudo-coordinate ``edge_feature[e, 0]``, + x root + bias; loops kept, none added
 """
+import math
+
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -101,6 +105,59 @@ class _GATConvLayer(nn.Module):
         return F_.gat_aggregate(h, self.att, self.bias, layout, self.heads, self.negative_slope)
 
 
+class _SplineConvLayer(nn.Module):
+    """PyG 1.6 ``SplineConv`` for dim = 1, kernel_size = 2, degree = 1, open spline, aggr 'mean', root weight: with
+    t = trunc(u_e), fr = u_e - floor(u_e), edge e = (j -> i) weighs x_j by 1 - fr through kernel matrix t mod 2 and by fr
+    through (t + 1) mod 2 (a non-negative mod: for u_e <= -1, where the reference indexes weight[-1], this is the
+    continuation of the pattern it has for u_e > -1).  out_i = mean_e (...) + x_i root + bias; a row without in-edges gets
+    x_i root + bias.  The other settings of the reference class are refused."""
+
+    def __init__(self, in_channels, out_channels, dim=1, kernel_size=2, is_open_spline=True, degree=1, bias=True):
+        super().__init__()
+        if dim != 1 or kernel_size != 2 or degree != 1 or not is_open_spline:
+            raise NotImplementedError('SplineConv: only dim=1, kernel_size=2, degree=1 with an open spline are on the '
+                                      'accelerated path (got dim={}, kernel_size={}, degree={}, is_open_spline={})'.format(
+                                          dim, kernel_size, degree, is_open_spline))
+        self.in_channels, self.out_channels = in_channels, out_channels
+        self.register_buffer('kernel_size', torch.tensor([kernel_size], dtype=torch.long))
+        self.register_buffer('is_open_spline', torch.tensor([1], dtype=torch.uint8))
+        self.weight = Parameter(torch.empty(kernel_size, in_channels, out_channels))
+        self.root = Parameter(torch.empty(in_channels, out_channels))
+        if bias:
+            self.bias = Parameter(torch.empty(out_channels))
+        else:
+            self.register_parameter('bias', None)
+        self.reset_parameters()
+
+    def reset_parameters(self):
+        bound = 1.0 / math.sqrt(self.weight.size(0) * self.weight.size(1))     # PyG's uniform(size, t)
+        for t in (self.weight, self.root, self.bias):
+            if t is not None:
+                with torch.no_grad():
+                    t.uniform_(-bound, bound)
+
+    def forward(self, x, edge_index, pseudo):
+        e = edge_index.size(1)
+        if pseudo is None:
+            raise ValueError('edge_feature: splineconv needs the pseudo-coordinates batch.edge_feature ([E] or [E, 1])')
+        if pseudo.dtype != torch.float32:
+            raise ValueError('edge_feature: splineconv needs float32 pseudo-coordinates, got {}'.format(pseudo.dtype))
+        if pseudo.dim() == 2 and pseudo.size(1) != 1:
+            raise ValueError('edge_feature: splineconv has dim=1 (one pseudo-coordinate per edge), got {}; PyG\'s dim=1 '
+                             'basis would read out of bounds on a wider edge_feature'.format(tuple(pseudo.shape)))
+        if pseudo.dim() not in (1, 2) or pseudo.size(0) != e:
+            raise ValueError('edge_feature: expected [{}] or [{}, 1] pseudo-coordinates, got {}'.format(
+                e, e, tuple(pseudo.shape)))
+        if cfg.b200.gather_dtype == 'bf16':
+            raise NotImplementedError("cfg.b200.gather_dtype = 'bf16' has no splineconv aggregation")
+        layout = get_layout(edge_index, x.size(0), ops.LOOPS_KEEP)
+        return F_.spline_aggregate(x, pseudo, self.weight, self.root, self.bias, layout,
+                                   self.in_channels <= self.out_channels)
+
+    def __repr__(self):
+        return '{}({}, {}, dim=1)'.format(self.__class__.__name__, self.in_channels, self.out_channels)
+
+
 class _EdgeIndexWrapper(nn.Module):
     def forward(self, batch):
         batch.node_feature = self.model(batch.node_feature, batch.edge_index)
@@ -130,6 +187,19 @@ class GINConv(_EdgeIndexWrapper):
         super().__init__()
         gin_nn = nn.Sequential(nn.Linear(dim_in, dim_out), nn.ReLU(), nn.Linear(dim_out, dim_out))
         self.model = _GINConvLayer(gin_nn)
+
+
+class SplineConv(nn.Module):
+    """ref: graphgym/models/layer.py, SplineConv: pyg.nn.SplineConv(dim_in, dim_out, dim=1, kernel_size=2) over
+    (node_feature, edge_index, edge_feature); cfg.gnn.agg / normalize_adj are not read."""
+
+    def __init__(self, dim_in, dim_out, bias=False, **kwargs):
+        super().__init__()
+        self.model = _SplineConvLayer(dim_in, dim_out, dim=1, kernel_size=2, bias=bias)
+
+    def forward(self, batch):
+        batch.node_feature = self.model(batch.node_feature, batch.edge_index, batch.edge_feature)
+        return batch
 
 
 _ACT = {'relu': nn.ReLU, 'selu': nn.SELU, 'prelu': nn.PReLU, 'elu': nn.ELU,
@@ -196,6 +266,7 @@ _builtin = {
     'generalconv': _generalconv.GeneralConv,
     'generaledgeconv': _generalconv.GeneralEdgeConv,
     'generalsampleedgeconv': _generalconv.GeneralSampleEdgeConv,
+    'splineconv': SplineConv,
 }
 
 # built-ins win on a name clash, contrib registrations fill the rest (ref: layer.py:238)

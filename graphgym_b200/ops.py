@@ -598,6 +598,99 @@ def edge_max_wgrad(csr, arg, g, a):
     return dw
 
 
+def _spline_u(u, csr):
+    if u.dtype != torch.float32 or u.dim() != 1 or u.numel() != csr.num_edges:
+        raise ValueError(f"pseudo-coordinates: expected a [{csr.num_edges}] float32 tensor, got {tuple(u.shape)} {u.dtype}")
+    return u.contiguous()
+
+
+def _spline_algo(csr, f, lds, tensors, algo, name):
+    aligned = f % 4 == 0 and all(ld % 4 == 0 for ld in lds) and all(_al16(t) for t in tensors)
+    if algo is None:
+        algo = "sell" if aligned and csr.num_nodes + csr.num_slots >= 1 << 14 else "row"
+    if algo == "sell" and not aligned:
+        raise ValueError(f"{name}: the sliced-ELL kernel needs f % 4 == 0 and 16-byte aligned rows")
+    if algo not in ("sell", "row"):
+        raise ValueError(f"{name}: algo={algo!r}")
+    return algo
+
+
+def spline_spread(csr, x, u, w_slot=None, mean=False, algo=None):
+    """[n, 2f] = [sum_s w_s c0_s x[nbr[s]] | sum_s w_s c1_s x[nbr[s]]] per row (/ indeg with ``mean``), (c0, c1) the
+    degree-1 open B-spline coefficients of the pseudo-coordinate u[perm[s]] (kernel size 2; csrc/spline_agg.cu).
+    ``u``: [E] float32 in edge order; ``w_slot``: per-slot weights of ``csr`` or None.  Path choice as ``spmm_max``;
+    ``algo`` ('sell' | 'row') overrides it."""
+    _need_cuda(x, u, w_slot, csr.rowptr)
+    x, ldx = _rows(x, "x")
+    u = _spline_u(u, csr)
+    n, f = csr.num_nodes, x.size(1)
+    out = _f32((n, 2 * f), x.device)
+    if n == 0 or f == 0:
+        return out
+    L = lib()
+    if _spline_algo(csr, f, (ldx,), (x,), algo, "spline_spread") == "sell":
+        sl = sell_layout(csr)
+        ws_bytes = int(L.gg_spmm_sell_max_workspace_bytes(sl.partial_rows, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        check(L.gg_spline_spread_sell_f32(_ptr(sl.chunk_ptr), sl.chunks, _ptr(sl.idx), _ptr(sl.slot_of),
+                                          _ptr(sl.weights(w_slot)), _ptr(csr.perm), _ptr(u), _ptr(sl.vdst), _ptr(csr.rowptr),
+                                          _ptr(sl.hub_rows), _ptr(sl.hub_pptr), sl.hubs, sl.partial_rows, _ptr(x), ldx,
+                                          _ptr(out), 2 * f, n, f, int(bool(mean)), _ptr(ws), ws_bytes, _spmm_flags(),
+                                          _stream()), "gg_spline_spread_sell_f32")
+    else:
+        check(L.gg_spline_spread_row_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(csr.perm), _ptr(w_slot), _ptr(u), _ptr(x), ldx,
+                                         _ptr(out), 2 * f, n, f, int(bool(mean)), _stream()), "gg_spline_spread_row_f32")
+    return out
+
+
+def spline_blend(csr, y, u, w_slot=None, mean=False, residual=None, bias=None, algo=None):
+    """[n, f]: sum_s w_s (c0_s y[nbr[s], :f] + c1_s y[nbr[s], f:]) per row (/ indeg with ``mean``) + residual + bias;
+    ``y``: [*, 2f].  Coefficients, ``u``, ``w_slot`` and the path choice as ``spline_spread``."""
+    _need_cuda(y, u, w_slot, residual, bias, csr.rowptr)
+    y, ldy = _rows(y, "y")
+    u = _spline_u(u, csr)
+    n, f = csr.num_nodes, y.size(1) // 2
+    if y.size(1) != 2 * f:
+        raise ValueError(f"spline_blend: y must have an even width, got {tuple(y.shape)}")
+    out = _f32((n, f), y.device)
+    if n == 0 or f == 0:
+        return out
+    ld_res = 0
+    if residual is not None:
+        residual, ld_res = _rows(residual, "residual")
+    if bias is not None:
+        bias = bias.contiguous()
+    L = lib()
+    if _spline_algo(csr, f, (ldy, ld_res), (y, residual, bias), algo, "spline_blend") == "sell":
+        sl = sell_layout(csr)
+        ws_bytes = int(L.gg_spmm_sell_max_workspace_bytes(sl.partial_rows, f))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=y.device)
+        check(L.gg_spline_blend_sell_f32(_ptr(sl.chunk_ptr), sl.chunks, _ptr(sl.idx), _ptr(sl.slot_of),
+                                         _ptr(sl.weights(w_slot)), _ptr(csr.perm), _ptr(u), _ptr(sl.vdst), _ptr(csr.rowptr),
+                                         _ptr(sl.hub_rows), _ptr(sl.hub_pptr), sl.hubs, sl.partial_rows, _ptr(y), ldy,
+                                         _ptr(out), f, n, f, int(bool(mean)), _ptr(residual), ld_res, _ptr(bias), _ptr(ws),
+                                         ws_bytes, _spmm_flags(), _stream()), "gg_spline_blend_sell_f32")
+    else:
+        check(L.gg_spline_blend_row_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(csr.perm), _ptr(w_slot), _ptr(u), _ptr(y), ldy,
+                                        _ptr(out), f, n, f, int(bool(mean)), _ptr(residual), ld_res, _ptr(bias), _stream()),
+              "gg_spline_blend_row_f32")
+    return out
+
+
+def spline_du(csr, u, a, a_half, b, b_half, f):
+    """[E] in edge order: du[perm[s]] = (dc[(t+1) mod 2] - dc[t mod 2]) / indeg(i) for the slots s of row i, t = trunc(u),
+    dc_k = <a[i, k a_half : k a_half + f], b[nbr[s], k b_half : k b_half + f]> (a_half / b_half = 0: one operand for both
+    matrices) — the pseudo-coordinate gradient of the mean B-spline aggregation."""
+    _need_cuda(u, a, b, csr.rowptr)
+    a, lda = _rows(a, "a")
+    b, ldb = _rows(b, "b")
+    u = _spline_u(u, csr)
+    du = _f32((csr.num_edges,), u.device)
+    check(lib().gg_spline_du_f32(_ptr(csr.rowptr), _ptr(csr.nbr), _ptr(csr.perm), _ptr(u), _ptr(a), lda, int(a_half),
+                                 _ptr(b), ldb, int(b_half), csr.num_nodes, int(f), _ptr(du), _stream()), "gg_spline_du_f32")
+    return du
+
+
 def rows_epilogue(x, mean_csr=None, rank1=None, heads=1, bias=None, out=None):
     """out[i, :] = x[i, :] / indeg(i) (with ``mean_csr``; rows without in-edges unscaled) + s1[i, k] v1 + s2[i, k] v2
     (``rank1`` = (s1 [n, heads], v1 [f], s2, v2), k the column's head) + bias.  ``out`` may be ``x``."""

@@ -312,6 +312,43 @@ int gg_edge_max_wgrad_f32(const int32_t* perm, const int32_t* arg, int64_t ld_ar
                           const float* a, int64_t lda, int64_t num_rows, int64_t f, int64_t kd, float* dw, int64_t lddw,
                           void* workspace, size_t workspace_bytes, gg_stream_t stream);
 
+/* B-spline weighted mean aggregation (csrc/spline_agg.cu; splineconv, degree 1, kernel size 2, open spline).  Slot s of
+ * row i gathers row nbr[s]; its edge perm[s] has pseudo-coordinate u[perm[s]], t = trunc(u), fr = u - floor(u), and the
+ * coefficients c[t & 1] = 1 - fr, c[(t & 1) ^ 1] = fr (t & 1: the non-negative t mod 2).  w_s = w_slot[s] (nullable: 1);
+ * `mean` divides row i by its slot count (rows without slots: 0 + the epilogue terms).
+ *   gg_spline_spread_*_f32    out[i, 0:f] = sum_s w_s c0 x[nbr[s], :], out[i, f:2f] = sum_s w_s c1 x[nbr[s], :]
+ *   gg_spline_blend_*_f32     out[i, :] = sum_s w_s (c0 y[nbr[s], 0:f] + c1 y[nbr[s], f:2f]) + res[i, :] + bias
+ *                             (res, bias nullable)
+ *                             Slot order per row.  The sliced-ELL entries take the layout's gg_sell_build arrays (slot_of
+ *                             gives the slot of every entry, w_sell the weights re-laid by gg_sell_permute_f32, flags bit 2
+ *                             as in gg_spmm_sell_f32), f % 4 == 0 (GG_ERR_UNSUPPORTED otherwise), 16-byte aligned rows,
+ *                             workspace gg_spmm_sell_max_workspace_bytes(partial rows, f); the row entries take the plain
+ *                             layout and any f.
+ *   gg_spline_du_f32          du[perm[s]] = (dc[(t+1) & 1] - dc[t & 1]) / indeg(i) for every slot s of row i, with
+ *                             dc_k = sum_{c < f} a[i, k a_half + c] b[nbr[s], k b_half + c] (a_half / b_half = 0: one
+ *                             operand for both k).  One warp per row, fixed reduction order.
+ * All are bitwise run-to-run deterministic (no atomics on data). */
+int gg_spline_spread_sell_f32(const uint32_t* chunk_ptr, int64_t chunks, const int32_t* idx, const int32_t* slot_of,
+                              const float* w_sell, const int32_t* perm, const float* u, const int32_t* vdst,
+                              const int32_t* rowptr, const int32_t* hub_rows, const int32_t* hub_pptr, int64_t hubs,
+                              int64_t partial_rows, const float* x, int64_t ldx, float* out, int64_t ldo, int64_t num_rows,
+                              int64_t f, int mean, void* workspace, size_t workspace_bytes, int flags, gg_stream_t stream);
+int gg_spline_blend_sell_f32(const uint32_t* chunk_ptr, int64_t chunks, const int32_t* idx, const int32_t* slot_of,
+                             const float* w_sell, const int32_t* perm, const float* u, const int32_t* vdst,
+                             const int32_t* rowptr, const int32_t* hub_rows, const int32_t* hub_pptr, int64_t hubs,
+                             int64_t partial_rows, const float* y, int64_t ldy, float* out, int64_t ldo, int64_t num_rows,
+                             int64_t f, int mean, const float* res, int64_t ld_res, const float* bias, void* workspace,
+                             size_t workspace_bytes, int flags, gg_stream_t stream);
+int gg_spline_spread_row_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* perm, const float* w_slot,
+                             const float* u, const float* x, int64_t ldx, float* out, int64_t ldo, int64_t num_rows,
+                             int64_t f, int mean, gg_stream_t stream);
+int gg_spline_blend_row_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* perm, const float* w_slot,
+                            const float* u, const float* y, int64_t ldy, float* out, int64_t ldo, int64_t num_rows,
+                            int64_t f, int mean, const float* res, int64_t ld_res, const float* bias, gg_stream_t stream);
+int gg_spline_du_f32(const int32_t* rowptr, const int32_t* nbr, const int32_t* perm, const float* u, const float* a,
+                     int64_t lda, int64_t a_half, const float* b, int64_t ldb, int64_t b_half, int64_t num_rows, int64_t f,
+                     float* du, gg_stream_t stream);
+
 /* Mean / max aggregation of the attention layers (csrc/attn_agg.cu; gaddconv / gmulconv with cfg.gnn.agg = 'mean' /
  * 'max').  heads H splits f into H blocks of c = f / H columns; column col belongs to head col / c.
  *   gg_max_winner_sddmm_f32   dalpha[s*H + k] = sum over the columns col of head k with arg[i,col] == s (s a slot of CSR
